@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the FLowHigh `generate` hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): midpoint ODE (2 NFE), batch of 64 x 10 s clips, 12 kHz -> 48 kHz,
 basic_cfm, transformer 2L x 16H x 64, BigVGAN 48 kHz / 256-band (ASSUMED vocoder config, SURVEY A.6),
@@ -17,6 +17,10 @@ whole path (resample -> log-mel -> CFM -> vocoder -> post-processing) over one b
 
 N > 1: launched by torchrun, one rank per GPU, each rank runs its own batch (weak scaling, clips are
 independent: no data-path collective); time = max over ranks.
+
+--dump-outputs DIR: after the timed steps, rank 0 writes the waveforms its last timed step returned as
+DIR/audio.npy (float32).  Inputs, noise and weights come from fixed seeds, so two builds run with the same
+arguments can be compared output for output; an output above DUMP_BYTES is cut to a fixed seeded sample.
 """
 from __future__ import annotations
 
@@ -40,6 +44,7 @@ CLIP_SECONDS = 10.0
 SR_IN = 12000
 BATCH = 64
 STEPS_ODE = 1  # time_step = 1, midpoint -> 2 NFE
+DUMP_BYTES = 48 << 20  # --dump-outputs: bound on what one run writes (batch64 at B = 64: 26 of the 64 clips)
 
 
 def config_dict(n_gpus, batch):
@@ -108,6 +113,24 @@ class ClockSampler:
                 "sm_mhz_min": min(sm) if sm else None, "sm_mhz_peak": max(sm) if sm else None,
                 "reasons": reasons, "samples": len(sm), "power_w": statistics.median(pw) if pw else None,
                 "power_limit_w": max(pl) if pl else None}
+
+
+def dump_outputs(path, name, out):
+    """Writes `out` as <path>/<name>.npy in float32.  Above DUMP_BYTES, whole rows (clips) drawn with a fixed seed
+    are kept, in ascending order; a single row longer than that is cut to fixed seeded sample positions instead."""
+    import torch
+    a = out.detach().float()
+    if a.numel() * 4 > DUMP_BYTES:
+        rng = np.random.default_rng(0)
+        row = a[0].numel() * 4
+        if a.shape[0] > 1 and row <= DUMP_BYTES:
+            idx = np.sort(rng.choice(a.shape[0], DUMP_BYTES // row, replace=False))
+        else:
+            a = a.flatten()
+            idx = np.sort(rng.choice(a.numel(), DUMP_BYTES // 4, replace=False))
+        a = a[torch.from_numpy(idx).to(a.device)]
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, name + ".npy"), a.cpu().numpy())
 
 
 # ------------------------------------------------------------------------------------------- CPU arm
@@ -289,6 +312,8 @@ def run_sharded_workload(args, model, eng, dev, world, rank, local):
     finite = bool(torch.isfinite(out).all())
     if not finite:
         raise RuntimeError("bench: non-finite output")
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, "audio", out)
     if rank == 0:
         total = sum(ts)
         med = statistics.median(ts)
@@ -329,7 +354,14 @@ def main():
                          "ncclAllGather); longform = configs[3]: one 10-minute clip, overlapped chunks over the ranks + overlap-add")
     ap.add_argument("--clips", type=int, default=512, help="mixed512: total number of clips")
     ap.add_argument("--minutes", type=float, default=10.0, help="longform: clip length")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned to DIR/audio.npy (float32, a fixed seeded sample above "
+                         f"{DUMP_BYTES >> 20} MiB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.impl == "reference" and args.dump_outputs:
+        ap.error("--dump-outputs applies to the GPU implementation")
     if args.impl == "reference":
         run_reference_arm(args)
         return
@@ -425,6 +457,8 @@ def main():
     if not finite or status:
         raise RuntimeError(f"bench: the timed step produced a non-finite output (finite={finite}) or tripped the 16-bit "
                            f"overflow guard (status {status:#x})")
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, "audio", out)
     self_check = None
     if rank == 0:
         model.cuda_graphs = False
@@ -441,7 +475,7 @@ def main():
     step_e2e()
     barrier()
     t0 = time.perf_counter()
-    e2e_steps = max(1, min(args.steps, 3))
+    e2e_steps = args.steps
     for _ in range(e2e_steps):
         step_e2e()
     barrier()

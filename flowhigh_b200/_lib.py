@@ -30,10 +30,8 @@ class TcConvArgs(C.Structure):
         ("tap_off", C.POINTER(_i)),
         ("bn", _i),
         ("fp16", _i),
-        ("x_f32", _p), ("sn_a", _p), ("sn_inv_b", _p), ("sn_filt", _p),
         ("act", _i),
         ("acc_src", _p),
-        ("x_is_16", _i),
         ("two_cta", _i),
     ]
 
@@ -50,12 +48,10 @@ SIGNATURES = {
     "fh_absmax_f32": (_i, [_p, _p, _i, _i, _p]),
     "fh_fill_u32": (_i, [_p, C.c_uint32, _i64, _p]),
     "fh_stft_logmel_f32": (_i, [_p, _p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _i, _p]),
-    "fh_stft_center_f32": (_i, [_p, _p, _p, _p, _p, _i, _i, _i, _p]),
     "fh_pp_cutoff": (_i, [_p, _p, _i, _f, _p]),
     "fh_pp_energy_ws_bytes": (_i, [_i, _i]),
     "fh_pp_src_energy_f32": (_i, [_p, _p, _p, _p, _p, _i, _i, _i, _p]),
     "fh_pp_fused_f32": (_i, [_p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _p]),
-    "fh_pp_splice_istft_f32": (_i, [_p, _p, _p, _p, _p, _p, _i, _i, _p]),
     "fh_pp_overlap_add_f32": (_i, [_p, _p, _p, _p, _i, _i, _i, _p]),
     "fh_ola_crossfade_f32": (_i, [_p, _p, _i, _i, _i, _i64, _p]),
     "fh_sgemm_nt_f32": (_i, [_p, _i, _p, _i, _p, _p, _i, _f, _f, _p, _i, _i, _i, _i, _p]),

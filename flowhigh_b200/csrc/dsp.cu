@@ -296,38 +296,6 @@ __global__ void __launch_bounds__(128) stft_logmel_kernel(const float* __restric
 }
 
 // ------------------------------------------------------------------------------ post-processing
-__global__ void __launch_bounds__(128) stft_center_kernel(const float* __restrict__ xin, float2* __restrict__ spec,
-                                                          const float* __restrict__ window,
-                                                          const float2* __restrict__ tw, int Tlen, int NT) {
-  __shared__ __align__(16) Cplx<float> sa[kFftBuf];
-  __shared__ __align__(16) Cplx<float> sb[kFftBuf];
-  const int n = blockIdx.x, bi = blockIdx.y;
-  const float* x = xin + (size_t)bi * Tlen;
-  for (int i = threadIdx.x; i < 2048; i += blockDim.x) {
-    const int pos = n * 480 + i - 1024;  // center=True, pad_mode='constant' (postprocessing.py:7)
-    const float v = (pos >= 0 && pos < Tlen) ? __ldg(x + pos) * __ldg(window + i) : 0.f;
-    sa[i] = {v, 0.f};
-  }
-  __syncthreads();
-  Cplx<float>* r = fft2048<float, false>(sa, sb, tw);
-  float2* out = spec + ((size_t)bi * NT + n) * 1025;
-  for (int f = threadIdx.x; f <= 1024; f += blockDim.x) out[f] = make_float2(r[f].x, r[f].y);
-}
-
-// energy[b,f] = sum_t |S[b,t,f]|  (fixed order -> deterministic cutoff)
-__global__ void pp_energy_kernel(const float2* __restrict__ spec, float* __restrict__ energy, int NT) {
-  const int bi = blockIdx.y;
-  const int f = blockIdx.x * blockDim.x + threadIdx.x;
-  if (f > 1024) return;
-  const float2* s = spec + (size_t)bi * NT * 1025 + f;
-  double acc = 0.0;
-  for (int t = 0; t < NT; ++t) {
-    const float2 v = s[(size_t)t * 1025];
-    acc += (double)hypotf(v.x, v.y);
-  }
-  energy[(size_t)bi * 1025 + f] = (float)acc;
-}
-
 __global__ void pp_cutoff_kernel(const float* __restrict__ energy, int* __restrict__ cutoff, float threshold) {
   // sequential fp32 cumsum like torch.cumsum on CPU; scan from the top, never testing bin 0
   __shared__ float cum[1025];
@@ -347,28 +315,6 @@ __global__ void pp_cutoff_kernel(const float* __restrict__ energy, int* __restri
       }
     cutoff[bi] = cr;
   }
-}
-
-__global__ void __launch_bounds__(128) pp_splice_istft_kernel(const float2* __restrict__ sp, const float2* __restrict__ ss,
-                                                              const int* __restrict__ cutoff, float* __restrict__ frames,
-                                                              const float* __restrict__ window,
-                                                              const float2* __restrict__ tw, int NT) {
-  __shared__ __align__(16) Cplx<float> sa[kFftBuf];
-  __shared__ __align__(16) Cplx<float> sb[kFftBuf];
-  const int n = blockIdx.x, bi = blockIdx.y;
-  const int cr = cutoff[bi];
-  const size_t base = ((size_t)bi * NT + n) * 1025;
-  for (int k = threadIdx.x; k < 2048; k += blockDim.x) {
-    const int f = k <= 1024 ? k : 2048 - k;
-    float2 v = f < cr ? ss[base + f] : sp[base + f];
-    if (f == 0 || f == 1024) v.y = 0.f;  // c2r ignores the imaginary part of DC / Nyquist
-    if (k > 1024) v.y = -v.y;
-    sa[k] = {v.x, v.y};
-  }
-  __syncthreads();
-  Cplx<float>* r = fft2048<float, true>(sa, sb, tw);
-  float* out = frames + ((size_t)bi * NT + n) * 2048;
-  for (int i = threadIdx.x; i < 2048; i += blockDim.x) out[i] = r[i].x * (1.0f / 2048.0f) * __ldg(window + i);
 }
 
 // ---- fused post-processing: no spectrogram ever reaches HBM ------------------------------------------------------
@@ -564,18 +510,6 @@ extern "C" __attribute__((visibility("default"))) int fh_stft_logmel_f32(const f
   return fh::check_launch("fh_stft_logmel_f32");
 }
 
-extern "C" __attribute__((visibility("default"))) int fh_stft_center_f32(const float* x, float* spec, float* energy, const float* window,
-                                  const float* twiddle, int B, int T, int NT, void* stream) {
-  FH_REQUIRE(B > 0 && T > 0 && NT == 1 + T / 480, FH_ERR_BAD_SHAPE, "fh_stft_center_f32: NT=%d does not match T=%d", NT,
-             T);
-  stft_center_kernel<<<dim3(NT, B), 128, 0, (cudaStream_t)stream>>>(x, (float2*)spec, window, (const float2*)twiddle, T,
-                                                                    NT);
-  int rc = fh::check_launch("fh_stft_center_f32");
-  if (rc != FH_OK || !energy) return rc;
-  pp_energy_kernel<<<dim3((1025 + 127) / 128, B), 128, 0, (cudaStream_t)stream>>>((const float2*)spec, energy, NT);
-  return fh::check_launch("fh_stft_center_f32(energy)");
-}
-
 extern "C" __attribute__((visibility("default"))) int fh_pp_cutoff(const float* energy, int* cutoff, int B, float threshold, void* stream) {
   FH_REQUIRE(B > 0, FH_ERR_BAD_SHAPE, "fh_pp_cutoff: bad shape");
   pp_cutoff_kernel<<<B, 32, 0, (cudaStream_t)stream>>>(energy, cutoff, threshold);
@@ -611,14 +545,6 @@ extern "C" __attribute__((visibility("default"))) int fh_pp_fused_f32(const floa
   pp_fused_kernel<<<dim3(NT, B), 128, 0, (cudaStream_t)stream>>>(pred, src, cutoff, frames, window, (const float2*)twiddle, Tp,
                                                                 T, NT);
   return fh::check_launch("fh_pp_fused_f32");
-}
-
-extern "C" __attribute__((visibility("default"))) int fh_pp_splice_istft_f32(const float* spec_pred, const float* spec_src, const int* cutoff, float* frames,
-                                      const float* window, const float* twiddle, int B, int NT, void* stream) {
-  FH_REQUIRE(B > 0 && NT > 0, FH_ERR_BAD_SHAPE, "fh_pp_splice_istft_f32: bad shape");
-  pp_splice_istft_kernel<<<dim3(NT, B), 128, 0, (cudaStream_t)stream>>>(
-      (const float2*)spec_pred, (const float2*)spec_src, cutoff, frames, window, (const float2*)twiddle, NT);
-  return fh::check_launch("fh_pp_splice_istft_f32");
 }
 
 extern "C" __attribute__((visibility("default"))) int fh_pp_overlap_add_f32(const float* frames, float* y, const float* window, uint32_t* absmax_bits, int B,

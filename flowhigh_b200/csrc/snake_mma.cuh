@@ -14,8 +14,7 @@
 //   * snake on the accumulator registers (packed FMUL2 / FFMA2, MUFU.COS);
 //   * two adjacent accumulator tiles of the up stage ARE the A fragment of the down stage (16 up-samples), so
 //     nothing is shuffled or staged:  Y[seq][8 outputs] = sum_{d=-1,0,1} S_{i+d}[seq][16] . Tdn_d[16][8];
-//   * the filter taps are fp16, chosen by error feedback inside each polyphase branch (exact DC gains); SPLIT_F keeps
-//     the exact taps as hi + lo pairs (extra MMAs);
+//   * the filter taps are fp16, chosen by error feedback inside each polyphase branch (exact DC gains);
 //   * the output tile goes to shared memory with stmatrix.trans ([time][8 ch] rows) and to HBM with one bulk store.
 // Replicate clamps: x~ is patched in the shared-memory window (first / last segments); the s~ clamp only changes the
 // first and last three outputs of a sequence, which the warp recomputes in scalar fp32 on those segments.
@@ -41,9 +40,8 @@ struct SnakeMmaGeom {
   static constexpr int kXBytes = kXRows * 32;  // fp32 rows; fp16 input rows take half of it
   static constexpr int kWarpYBytes = kWarpRows * 16;
   // two input windows, per warp two output images, 128 control bytes: two mbarriers, two release counters, 2 x 12 taps
-  // wbuf input windows (2 = double buffered; 1 = single: a third CTA fits per SM and the other CTAs cover the refill)
-  static constexpr int smem_bytes(bool in16, bool split_out = false, int wbuf = 2) {
-    return wbuf * (in16 ? kXBytes / 2 : kXBytes) + (split_out ? 4 : 2) * kWarps * kWarpYBytes + 128;
+  static constexpr int smem_bytes(bool in16, bool split_out = false) {
+    return 2 * (in16 ? kXBytes / 2 : kXBytes) + (split_out ? 4 : 2) * kWarps * kWarpYBytes + 128;
   }
 };
 
@@ -73,7 +71,7 @@ __device__ __forceinline__ void sm_mma_k8(float (&d)[4], uint32_t a0, uint32_t a
                : "r"(a0), "r"(a1), "r"(b0), "f"(c0), "f"(c1), "f"(c2), "f"(c3));
 }
 
-// ---- pieces shared by the standalone kernel (snake_mma_cta) and the fused conv prologue (tc_conv.cu) ----------------
+// ---- pieces of snake_mma_cta -------------------------------------------------------------------------------------------
 
 // fp16 taps by ERROR FEEDBACK instead of round-to-nearest (one thread): within each polyphase branch (even / odd taps)
 // the taps are rounded in order of decreasing magnitude and every rounding error is carried into the next, finer-grained
@@ -82,7 +80,6 @@ __device__ __forceinline__ void sm_mma_k8(float (&d)[4], uint32_t a0, uint32_t a
 // s_taps[0, 12): up-filter taps (2 f), [12, 24): down-filter taps (f).
 // Four independent (filter, polyphase branch) chains: called by threads 0..3 with part = thread index (the serial form cost
 // ~3 us at the start of every launch -- a tenth of a B = 1 snake launch).
-template <bool SPLIT_F>
 __device__ __forceinline__ void snake_mma_make_taps(const float* __restrict__ filt, float* s_taps, int part) {
   const int w = part >> 1, ph = part & 1;
   const float scale = w ? 1.0f : 2.0f;
@@ -105,7 +102,7 @@ __device__ __forceinline__ void snake_mma_make_taps(const float* __restrict__ fi
 #pragma unroll
     for (int c = 1; c < 6; ++c) fb = best == c ? f[c] : fb;
     const float v = scale * fb + carry;
-    const float h = SPLIT_F ? v : __half2float(__float2half_rn(v));  // the tap-split mode keeps exact taps
+    const float h = __half2float(__float2half_rn(v));
     carry = v - h;
     s_taps[12 * w + 2 * best + ph] = h;
   }
@@ -113,7 +110,7 @@ __device__ __forceinline__ void snake_mma_make_taps(const float* __restrict__ fi
 
 // Toeplitz B fragments (k16 x n8, "col") of one thread: reg r holds k-slots 2q + 8r, 2q + 8r + 1 of column n = g
 struct SnakeFrags {
-  uint32_t bu[2][2], bul[2][2], bd[3][2], bdl[3][2];
+  uint32_t bu[2][2], bd[3][2];
 };
 template <bool IN16>
 __device__ __forceinline__ void snake_mma_frags(const float* s_taps, int lane, SnakeFrags& F) {
@@ -131,7 +128,7 @@ __device__ __forceinline__ void snake_mma_frags(const float* s_taps, int lane, S
     for (int r = 0; r < 2; ++r) {
       const int ko0 = IN16 ? 2 * q + 8 * r : q + 8 * r, ko1 = IN16 ? ko0 + 1 : ko0 + 4;
       const float v0 = tap(g + base - 2 * ko0, 2.0f), v1 = tap(g + base - 2 * ko1, 2.0f);
-      sm_split(v0, v1, F.bu[e][r], F.bul[e][r]);
+      F.bu[e][r] = sm_pack(v0, v1);
     }
   }
 #pragma unroll
@@ -141,7 +138,7 @@ __device__ __forceinline__ void snake_mma_frags(const float* s_taps, int lane, S
     for (int r = 0; r < 2; ++r) {
       const int c0 = 2 * q + 8 * r;
       const float v0 = tap(16 * (d - 1) + c0 - 2 * g + 5, 1.0f), v1 = tap(16 * (d - 1) + c0 + 1 - 2 * g + 5, 1.0f);
-      sm_split(v0, v1, F.bd[d][r], F.bdl[d][r]);
+      F.bd[d][r] = sm_pack(v0, v1);
     }
   }
 }
@@ -155,7 +152,7 @@ __device__ __forceinline__ void snake_mma_frags(const float* s_taps, int lane, S
 // clamped signal (finite) and must be ignored / overwritten by the caller.
 // SPLIT_OUT: the fp32 result is written as hi + lo fp16 pairs (yt_lo: second image, same geometry) -- the operand of a
 // convolution whose input channels are doubled [hi | lo] against duplicated weights keeps ~22 bits of the activation.
-template <bool SPLIT_X, bool SPLIT_F, int NB, bool IN16, bool SPLIT_OUT = false>
+template <bool SPLIT_X, int NB, bool IN16, bool SPLIT_OUT = false>
 __device__ __forceinline__ void snake_mma_unit(const SnakeFrags& F, float* xw, unsigned char* yt, int q0, int L, int ch,
                                                const float* __restrict__ sn_a, const float* __restrict__ sn_inv_b,
                                                const float* __restrict__ sn_filt, bool edge, int lo, int hi, int lane,
@@ -211,13 +208,11 @@ __device__ __forceinline__ void snake_mma_unit(const SnakeFrags& F, float* xw, u
                      : "=r"(a0), "=r"(a1), "=r"(a2), "=r"(a3)
                      : "r"(lm_base + (uint32_t)(k0 * 16)));
         sm_mma(dd, a0, a1, a2, a3, F.bu[e][0], F.bu[e][1], 0.f, 0.f, 0.f, 0.f);
-        if (SPLIT_F) sm_mma(dd, a0, a1, a2, a3, F.bul[e][0], F.bul[e][1], dd[0], dd[1], dd[2], dd[3]);
         return;
       }
       const int p = (e ? j : j - 1) + 1, n = p + 1;
       sm_mma(dd, xh[p][0], xh[p][1], xh[n][0], xh[n][1], F.bu[e][0], F.bu[e][1], 0.f, 0.f, 0.f, 0.f);
       if (SPLIT_X) sm_mma(dd, xl[p][0], xl[p][1], xl[n][0], xl[n][1], F.bu[e][0], F.bu[e][1], dd[0], dd[1], dd[2], dd[3]);
-      if (SPLIT_F) sm_mma(dd, xh[p][0], xh[p][1], xh[n][0], xh[n][1], F.bul[e][0], F.bul[e][1], dd[0], dd[1], dd[2], dd[3]);
     };
     auto snake2 = [&](float u0, float u1) -> uint32_t {
       const float2 u = make_float2(u0, u1);
@@ -259,25 +254,20 @@ __device__ __forceinline__ void snake_mma_unit(const SnakeFrags& F, float* xw, u
         float (&yy)[4] = y[(j - 1) % 3];
 #if FH_SNAKE_K8
         sm_mma_k8(yy, U[0], U[1], F.bd[2][0], yy[0], yy[1], yy[2], yy[3]);
-        if (SPLIT_F) sm_mma_k8(yy, U[0], U[1], F.bdl[2][0], yy[0], yy[1], yy[2], yy[3]);
 #else
         sm_mma(yy, U[0], U[1], U[2], U[3], F.bd[2][0], F.bd[2][1], yy[0], yy[1], yy[2], yy[3]);
-        if (SPLIT_F) sm_mma(yy, U[0], U[1], U[2], U[3], F.bdl[2][0], F.bdl[2][1], yy[0], yy[1], yy[2], yy[3]);
 #endif
       }
       if (j >= 0 && j < NB) {
         float (&yy)[4] = y[j % 3];
         sm_mma(yy, U[0], U[1], U[2], U[3], F.bd[1][0], F.bd[1][1], yy[0], yy[1], yy[2], yy[3]);
-        if (SPLIT_F) sm_mma(yy, U[0], U[1], U[2], U[3], F.bdl[1][0], F.bdl[1][1], yy[0], yy[1], yy[2], yy[3]);
       }
       if (j + 1 < NB) {  // first term of down block j + 1 (last 8 up-samples of step j)
         float (&yy)[4] = y[(j + 1) % 3];
 #if FH_SNAKE_K8
         sm_mma_k8(yy, U[2], U[3], F.bd[0][1], hib, hib, hib, hib);
-        if (SPLIT_F) sm_mma_k8(yy, U[2], U[3], F.bdl[0][1], yy[0], yy[1], yy[2], yy[3]);
 #else
         sm_mma(yy, U[0], U[1], U[2], U[3], F.bd[0][0], F.bd[0][1], hib, hib, hib, hib);
-        if (SPLIT_F) sm_mma(yy, U[0], U[1], U[2], U[3], F.bdl[0][0], F.bdl[0][1], yy[0], yy[1], yy[2], yy[3]);
 #endif
       }
       if (j >= 1) {
@@ -341,16 +331,16 @@ __device__ __forceinline__ void snake_mma_unit(const SnakeFrags& F, float* xw, u
 // IN16: the input is already fp16 on the same chunked layout (16-byte rows, written by the 16-bit epilogue of the
 // preceding convolution): the A fragments of the up stage come straight from the window with one ldmatrix.x4.trans
 // per 8 up-samples (identity k-slot -> time map), no conversion instructions at all.
-template <bool SPLIT_X, bool SPLIT_F, int NB, bool IN16 = false, bool SPLIT_OUT = false, int WBUF = 2>
+template <bool SPLIT_X, int NB, bool IN16 = false, bool SPLIT_OUT = false>
 __device__ __forceinline__ void snake_mma_cta(const SnakeParams& S, unsigned char* smem, int tid, int cta, int nctas) {
   using G = SnakeMmaGeom<NB>;
   const int lane = tid & 31, warp = tid >> 5;
   constexpr int kXB = IN16 ? G::kXBytes / 2 : G::kXBytes;  // bytes of one input window
   float* xs0 = reinterpret_cast<float*>(smem);
-  float* xs1 = reinterpret_cast<float*>(smem + (WBUF - 1) * kXB);
+  float* xs1 = reinterpret_cast<float*>(smem + kXB);
   constexpr int kImg = SPLIT_OUT ? 2 : 1;  // images per buffer (hi, lo)
-  unsigned char* ys0 = smem + WBUF * kXB + warp * 2 * kImg * G::kWarpYBytes;  // this warp's two output buffers
-  unsigned char* ctl = smem + WBUF * kXB + 2 * kImg * G::kWarps * G::kWarpYBytes;
+  unsigned char* ys0 = smem + 2 * kXB + warp * 2 * kImg * G::kWarpYBytes;  // this warp's two output buffers
+  unsigned char* ctl = smem + 2 * kXB + 2 * kImg * G::kWarps * G::kWarpYBytes;
   const uint32_t bar0 = sw_u32(ctl);
   int* released = reinterpret_cast<int*>(ctl + 16);  // warps done with window 0 / 1
   float* s_taps = reinterpret_cast<float*>(ctl + 32);  // [0, 12): up-filter taps (2 f), [12, 24): down-filter taps (f)
@@ -360,9 +350,9 @@ __device__ __forceinline__ void snake_mma_cta(const SnakeParams& S, unsigned cha
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     released[0] = released[1] = 0;
   }
-  if (tid < 4) snake_mma_make_taps<SPLIT_F>(S.filt, s_taps, tid);
+  if (tid < 4) snake_mma_make_taps(S.filt, s_taps, tid);
   // rows a clipped copy does not fill must hold finite values (they only ever meet zero filter weights)
-  for (int i = tid; i < WBUF * kXB / 16; i += 32 * G::kWarps) reinterpret_cast<float4*>(smem)[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+  for (int i = tid; i < 2 * kXB / 16; i += 32 * G::kWarps) reinterpret_cast<float4*>(smem)[i] = make_float4(0.f, 0.f, 0.f, 0.f);
   asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
   __syncthreads();
   const int rows_per_chunk = (int)(S.chunk_stride >> 3);
@@ -399,13 +389,11 @@ __device__ __forceinline__ void snake_mma_cta(const SnakeParams& S, unsigned cha
   Guard16 guard;
   int item = cta;
   int tile = item % S.ntile, ch = (item / S.ntile) % S.nchunk, b = (item / S.ntile) / S.nchunk;
-  int tile_f = tile, ch_f = ch, b_f = b;  // coordinates of the item WBUF steps ahead (the one a release refills)
+  int tile_f = tile, ch_f = ch, b_f = b;  // coordinates of the item two steps ahead (the one a release refills)
   if (tid == 0 && item < S.total) issue(tile, ch, b, 0);
   advance(tile_f, ch_f, b_f);
-  if (WBUF == 2) {
-    if (tid == 0 && item + nctas < S.total) issue(tile_f, ch_f, b_f, 1);
-    advance(tile_f, ch_f, b_f);
-  }
+  if (tid == 0 && item + nctas < S.total) issue(tile_f, ch_f, b_f, 1);
+  advance(tile_f, ch_f, b_f);
   int buf = 0, ybuf = 0;
   uint32_t ph0 = 0, ph1 = 0;
   const int ssA = warp * G::kWarpRows;  // first tile row of this warp's half A; half B starts kSeg rows later
@@ -419,8 +407,8 @@ __device__ __forceinline__ void snake_mma_cta(const SnakeParams& S, unsigned cha
     unsigned char* yt = ys0 + (size_t)ybuf * kImg * G::kWarpYBytes;
     if (active) {
       float* xw = reinterpret_cast<float*>(reinterpret_cast<unsigned char*>(xt) + (size_t)ssA * (IN16 ? 16 : 32));
-      snake_mma_unit<SPLIT_X, SPLIT_F, NB, IN16, SPLIT_OUT>(F, xw, yt, qt + ssA, S.L, ch, S.a, S.inv_b, S.filt, edge, -ssA,
-                                                            G::kXRows - ssA, lane, guard, yt + G::kWarpYBytes);
+      snake_mma_unit<SPLIT_X, NB, IN16, SPLIT_OUT>(F, xw, yt, qt + ssA, S.L, ch, S.a, S.inv_b, S.filt, edge, -ssA,
+                                                   G::kXRows - ssA, lane, guard, yt + G::kWarpYBytes);
     }
     // generic-proxy accesses of this warp (window reads / patches, output image writes) before the async proxy's
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
@@ -446,13 +434,13 @@ __device__ __forceinline__ void snake_mma_cta(const SnakeParams& S, unsigned cha
       if (atomicAdd(&released[buf], 1) == G::kWarps - 1) {
         released[buf] = 0;  // next touched after the refill below has landed and been consumed
         __threadfence_block();
-        if (item + WBUF * nctas < S.total) {
+        if (item + 2 * nctas < S.total) {
           asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
           issue(tile_f, ch_f, b_f, buf);
         }
       }
     }
-    if (WBUF == 2) buf ^= 1;
+    buf ^= 1;
     ybuf ^= 1;
   }
   if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");

@@ -1,7 +1,6 @@
 // Anti-aliased Snake / SnakeBeta on the chunked [C/8][Lp][8] layout as a *worker*: a group of 128 threads that walks
 // (batch, chunk, time-tile) work items with its own shared-memory buffers and named barrier.  The standalone kernel
-// (vocoder_tc.cu) is one worker per CTA; the dual kernel (tc_conv.cu) runs two workers beside the tcgen05 convolution
-// roles of another half-batch so that the FP32 pipe and the tensor pipe of an SM are busy at the same time.
+// (vocoder_tc.cu) is one worker per CTA.
 //
 // y[q] = sum_k f[k] s~[2q+k-5];  s[m] = u[m] + inv_b sin^2(a u[m]);  u[m] = 2 sum_i x~[i] f[m+5-2i]
 // (x~ / s~ = replicate-clamped; closed form of up2x -> snake -> down2x, SURVEY.md A.5; reference:

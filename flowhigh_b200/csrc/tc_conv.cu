@@ -18,10 +18,7 @@
 // reads them with tcgen05.ld.  Warp roles: warp 0 = bulk-copy producer, warp 1 = MMA issuer +
 // TMEM allocator, warps 2.. = epilogue (8 by default; 12 / 16 for the narrow HBM-bound shapes, whose
 // residual rows additionally stream through a per-warp cp.async ring).  Persistent CTAs, static tile striding.
-#include <stdlib.h>
 #include "common.cuh"
-#include "snake_worker.cuh"
-#include "snake_mma.cuh"
 #include "tc_ptx.cuh"
 
 namespace {
@@ -57,7 +54,9 @@ struct TcParams {
   int wrows;           // rows fetched per chunk window: 128*msub + (max_off - min_off)
   int arows_pad;       // rows reserved per chunk window in an A slot
   int stages, stage_bytes;
-  int empty_ring;       // number of "stage consumed" barriers the MMA issuer cycles through (= stages, or 8 in the fused kernel)
+  // empty_ring, m_stride and m_valid are always stages, 128 msub and 128 msub.  They stay fields: folding them into the
+  // kernels moves the spills of tc_conv_kernel<16> and the register count of tc_conv2_kernel.
+  int empty_ring;       // number of "stage consumed" barriers the MMA issuer cycles through
   int min_off[16];
   int tap_rel0[16];     // (offset of tap 0) - min_off of the phase
   int tap_step[16];     // offset(tap j+1) - offset(tap j) when the taps of a phase form an arithmetic sequence
@@ -71,13 +70,7 @@ struct TcParams {
   unsigned int* err_flag;
   unsigned int* status;  // overflow / NaN status word of the caller (common.cuh Guard16) or nullptr
   int two_cta;            // tc_conv2_kernel: CTA pairs share every weight slot (cta_group::2 MMA, M = 256)
-  int m_stride, m_valid;  // output rows a tile advances by / keeps (128 msub unless the A window is aligned: fused snake)
-  // fused anti-aliased snake prologue (tc_conv_snakepro_kernel): raw activations (fp32 or fp16 rows) + snake parameters
-  const void* xf;
-  const float* sn_a;
-  const float* sn_ib;
-  const float* sn_filt;
-  int x_stages, xs_bytes, xs_off, rows_per_chunk, pro_nb, snake_warps;
+  int m_stride, m_valid;  // output rows a tile advances by / keeps
 };
 
 
@@ -752,14 +745,13 @@ __device__ __forceinline__ void epilogue_dispatch(const TcParams& P, uint32_t tm
 
 // Per-CTA setup shared by the conv kernels: mbarriers, tap-offset table, alpha * bias table, zeroed partner windows.
 // The caller allocates TMEM and issues the __syncthreads that publishes all of it.
-__device__ __forceinline__ void conv_cta_setup(const TcParams& P, unsigned char* smem, int nthreads, int epi_warps,
-                                               int full_count = 1) {
+__device__ __forceinline__ void conv_cta_setup(const TcParams& P, unsigned char* smem, int nthreads, int epi_warps) {
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem);
   const uint32_t full0 = smem_u32(bars), empty0 = full0 + 8 * kMaxStages;
   const uint32_t tfull0 = empty0 + 8 * kMaxStages, tempty0 = tfull0 + 16;
   const int S = P.stages;
   if (threadIdx.x == 0) {
-    for (int i = 0; i < S; ++i) mbar_init(full0 + 8 * i, full_count);
+    for (int i = 0; i < S; ++i) mbar_init(full0 + 8 * i, 1);
     for (int i = 0; i < P.empty_ring; ++i) mbar_init(empty0 + 8 * i, 1);
     for (int i = 0; i < 2; ++i) {
       mbar_init(tfull0 + 8 * i, 1);
@@ -1022,207 +1014,6 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kThreads2, 1) tc_con
   }
 }
 
-// ------------------------------------------------------------------------------ fused snake prologue + conv
-// conv(Activation1d(x)) in ONE kernel for the HBM-bound stages (Cin <= 128, one N tile): the 16-bit activated operand
-// is produced in shared memory by eight "snake" warps running the Toeplitz-MMA snake (snake_mma.cuh) and consumed by
-// tcgen05.mma from there -- it never touches HBM (an AMPBlock1 unit drops from 24 to 16 bytes per element).
-//
-// Warp roles (20 warps): 0 = bulk-copy producer of raw activation windows (fp32 rows, or the fp16 rows the first
-// convolution of the unit wrote: IN16), 1 = MMA issuer + TMEM, 2 = bulk-copy producer of weight slots, 3 = idle,
-// 4..11 = epilogue (same specialised epilogues as tc_conv_kernel), 12..19 = snake warps.
-// One smem stage = one ci-pair (2 x 8 channels) x all taps; its A slot holds 128 msub window rows per chunk.
-// Work unit of a snake warp = 8 channels x 128 window rows (SnakeMmaGeom<8>): 2 chunks x msub units per stage.
-// Units are numbered globally (tile, chunk, sub); warp w takes units w, w + 8, ...; all synchronisation is by
-// mbarrier (x ring: one slot per unit window; stage full = weights landed + every unit of the stage written), so the
-// eight warps drift freely over several stages and never meet at a block barrier.
-// The A window is ALIGNED (exactly 128 msub rows starting at t0 + min_off): a tile therefore yields
-// m_valid = 128 msub - span output rows and tiles advance by m_valid rows; the discarded accumulator rows cost tensor
-// time these stages do not need, while the snake warps never compute a row twice within a tile.
-// Conv zero padding: image rows outside [0, L) are zeroed after the (replicate-clamped) snake wrote them.
-constexpr int kProThreads = 640;
-constexpr int kProSnakeWarps = 12;
-constexpr int kProEpiWarps = 4;
-constexpr int kProXMax = 24;  // x-ring slots
-
-// kProNB: snake unit = 8 channels x 16 kProNB window rows (128 or 256)
-template <bool IN16, int kProNB>
-__global__ void __launch_bounds__(kProThreads, 1) tc_conv_snakepro_kernel(const __grid_constant__ TcParams P) {
-  extern __shared__ __align__(1024) unsigned char smem[];
-  using G = fh::SnakeMmaGeom<kProNB>;
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem);
-  const uint32_t full0 = smem_u32(bars), empty0 = full0 + 8 * kMaxStages;
-  const uint32_t tfull0 = empty0 + 8 * kMaxStages, tempty0 = tfull0 + 16;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + 8 * (2 * kMaxStages + 4));
-  const uint32_t xfull0 = smem_u32(smem + P.xs_off + P.x_stages * P.xs_bytes), xempty0 = xfull0 + 8 * kProXMax;  // behind the x ring
-  int* s_off = reinterpret_cast<int*>(smem + 512);
-  float* s_taps = reinterpret_cast<float*>(smem + 768);
-  const uint32_t stage0 = smem_u32(smem + 1024);
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int S = P.stages, XD = P.x_stages;
-  const int h = (128 * P.msub) / G::kWarpRows;     // units per chunk and tile
-  const int AU = P.ci_pairs * 2 * h;               // units per tile, dummies of an odd last pair included
-  const int nchunks = P.Cin >> 3;
-  const int RU = nchunks * h;                      // real units (= x windows) per tile
-  constexpr uint32_t kRowB = IN16 ? 16u : 32u;
-  constexpr int kWinRows = G::kWarpRows + 2 * G::kHalo;  // 144
-  unsigned char* xring = smem + P.xs_off;
-  const uint32_t xwin_bytes = (uint32_t)P.xs_bytes;
-
-  conv_cta_setup(P, smem, kProThreads, kProEpiWarps, 1 + 2 * h);
-  if (threadIdx.x == 0) {
-    for (int i = 0; i < XD; ++i) {
-      mbar_init(xfull0 + 8 * i, 1);
-      mbar_init(xempty0 + 8 * i, 1);
-    }
-    fence_barrier_init();
-  }
-  if (threadIdx.x < 4) fh::snake_mma_make_taps<false>(P.sn_filt, s_taps, threadIdx.x);
-  // window rows a clipped copy does not fill, and the 64 spare rows behind every A window, must hold finite values
-  for (uint32_t i = threadIdx.x; i < (uint32_t)XD * xwin_bytes / 16u; i += kProThreads)
-    reinterpret_cast<uint4*>(xring)[i] = make_uint4(0u, 0u, 0u, 0u);
-  for (uint32_t i = threadIdx.x; i < (uint32_t)S * (uint32_t)P.stage_bytes / 16u; i += kProThreads)
-    reinterpret_cast<uint4*>(smem + 1024)[i] = make_uint4(0u, 0u, 0u, 0u);
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-  if (warp == 1) tmem_alloc(smem_u32(tmem_slot), 512);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  const uint32_t b_tap_bytes = (uint32_t)P.bn * 32u;
-  const uint32_t a_chunk_bytes = (uint32_t)P.arows_pad * 16u;
-  const uint32_t a_slot_bytes = 2u * a_chunk_bytes;
-  const uint32_t acc_cols = (uint32_t)(P.msub * P.bn);
-  const int mn = P.min_off[0];
-  // Stage sseq reuses the slot of stage sseq - S: wait until the MMAs of THAT stage have retired.  The issuer commits
-  // stage k to barrier k % 8, so a waiter would have to run 8 stages (>= 16 units) ahead of the issuer to alias a
-  // parity -- the eight snake warps cannot (each finishes unit u - 8 before it starts unit u).
-  auto wait_stage_free = [&](int sseq) {
-    if (sseq < S) return;
-    const int d = sseq - S;  // empty_ring == 8
-    mbar_wait(empty0 + 8 * (uint32_t)(d & 7), (uint32_t)((d >> 3) & 1), P.err_flag, 7);
-  };
-
-  if (warp < 4) {
-    asm volatile("setmaxnreg.dec.sync.aligned.u32 24;");
-    if (warp == 0) {
-      // ===================================================================== raw-activation window producer
-      if (lane == 0) {
-        int xs = 0;
-        uint32_t xph = 0;
-        for (int tile = blockIdx.x; tile < P.total_tiles; tile += gridDim.x) {
-          const TileCoord tc = decode_tile(P, tile);
-          const int t_slot0 = tc.mt * P.m_stride + mn;
-          const unsigned char* xb = reinterpret_cast<const unsigned char*>(P.xf) + (long long)tc.b * P.a_batch * (kRowB / 8);
-          for (int rv = 0; rv < RU; ++rv) {
-            const int chunk = rv / h, sub = rv - chunk * h;
-            mbar_wait(xempty0 + 8 * xs, xph ^ 1, P.err_flag, 5);
-            long long row = (long long)P.a_row0 + t_slot0 + sub * G::kWarpRows - G::kHalo;  // first window row in the chunk
-            int skip = row < 0 ? (int)(-row) : 0;                                          // rows before the buffer: replicate-patched
-            long long nrows = kWinRows - skip;
-            if (row + skip + nrows > P.rows_per_chunk) nrows = (long long)P.rows_per_chunk - row - skip;
-            const uint32_t fb = xfull0 + 8 * xs;
-            if (nrows > 0) {
-              mbar_expect_tx(fb, (uint32_t)nrows * kRowB);
-              bulk_g2s(smem_u32(xring) + (uint32_t)xs * xwin_bytes + (uint32_t)skip * kRowB,
-                       xb + ((long long)chunk * P.a_chunk + (row + skip) * 8) * (kRowB / 8), (uint32_t)nrows * kRowB, fb);
-            } else {
-              mbar_arrive(fb);
-            }
-            if (++xs == XD) {
-              xs = 0;
-              xph ^= 1;
-            }
-          }
-        }
-      }
-    } else if (warp == 2) {
-      // ===================================================================== weight producer
-      if (lane == 0) {
-        int stage = 0, sseq = 0;
-        for (int tile = blockIdx.x; tile < P.total_tiles; tile += gridDim.x) {
-          for (int cp = 0; cp < P.ci_pairs; ++cp, ++sseq) {
-            wait_stage_free(sseq);
-            const uint32_t sa = stage0 + (uint32_t)stage * (uint32_t)P.stage_bytes;
-            const uint32_t fb = full0 + 8 * stage;
-            mbar_expect_tx(fb, (uint32_t)P.ntaps * b_tap_bytes);
-            bulk_g2s(sa + a_slot_bytes, P.w + (long long)cp * P.ntaps * ((long long)P.bn * 16), (uint32_t)P.ntaps * b_tap_bytes, fb);
-            // odd last pair: its partner window (zeroed at setup, zero weights) has no snake units -- their arrivals are made here
-            if (P.ci_odd && cp == P.ci_pairs - 1) mbar_arrive_n(fb, (uint32_t)h);
-            if (++stage == S) stage = 0;
-          }
-        }
-      }
-    } else if (warp == 1) {
-      // ===================================================================== MMA issuer (one stage = one ci-pair)
-      mma_role(P, tmem_base, full0, empty0, tfull0, tempty0, stage0, a_chunk_bytes, s_off);
-    }
-  } else if (warp < 4 + kProEpiWarps) {
-    // ===================================================================== epilogue (4 warps, one per lane group: in
-    // this kernel the snake warps, not the epilogue, set the pace -- ncu: the epilogue warps wait for accumulators)
-    asm volatile("setmaxnreg.inc.sync.aligned.u32 120;");
-    epilogue_dispatch(P, tmem_base, tfull0, tempty0, warp & 3, 0, lane, P.m_stride, acc_cols,
-                      reinterpret_cast<const float*>(smem + 1024 + (size_t)P.stages * P.stage_bytes), 1);
-  } else {
-    // ===================================================================== snake warps
-    asm volatile("setmaxnreg.inc.sync.aligned.u32 112;");
-    const int sw = warp - 4 - kProEpiWarps;
-    if (sw >= P.snake_warps) goto done;  // (tiny shapes: fewer units per 8 stages than warps, see tc_plan)
-    fh::SnakeFrags F;
-    fh::snake_mma_frags<IN16>(s_taps, lane, F);
-    fh::Guard16 guard;
-    const int my_tiles = (P.total_tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
-    const int n_units = my_tiles * RU;  // < 2^31 (tc_plan)
-    // REAL units (= x windows) are dealt round-robin: warp w takes windows w, w + 8, ...  It has therefore consumed window
-    // n - 8 itself before it waits for window n, which keeps every parity wait below unambiguous (x ring of >= 8 slots
-    // filled in order; stage barriers cycling over 8 stages of >= 1 unit each).
-    for (int n = sw; n < n_units; n += P.snake_warps) {
-      const int tseq = n / RU, rv = n - tseq * RU;
-      const int chunk = rv / h, sub = rv - chunk * h;
-      const int pair = chunk >> 1, c = chunk & 1;
-      const int sseq = tseq * P.ci_pairs + pair;
-      const int slot = sseq % S;
-      const uint32_t fb = full0 + 8 * slot;
-      const int tile = (int)blockIdx.x + tseq * (int)gridDim.x;
-      const TileCoord tc = decode_tile(P, tile);
-      const int q0 = tc.mt * P.m_stride + mn + sub * G::kWarpRows;  // time of the unit's first image row
-      const int xg = n / XD, xs = n - xg * XD;
-      const uint32_t xph = (uint32_t)(xg & 1);
-      unsigned char* yt = smem + 1024 + (size_t)slot * P.stage_bytes + (size_t)c * a_chunk_bytes + (size_t)sub * G::kWarpYBytes;
-      mbar_wait(xfull0 + 8 * xs, xph, P.err_flag, 6);          // the raw window has landed
-      wait_stage_free(sseq);                                   // the MMAs that last read this A slot have retired
-      const bool active = q0 < P.L && q0 + G::kWarpRows > 0;
-      const bool edge = (q0 - G::kHalo < 0) || (q0 + G::kWarpRows + G::kHalo > P.L);
-      if (active) {
-        float* xw = reinterpret_cast<float*>(xring + (size_t)xs * xwin_bytes);
-        fh::snake_mma_unit<false, false, kProNB, IN16>(F, xw, yt, q0, P.L, chunk, P.sn_a, P.sn_ib, P.sn_filt, edge, 0,
-                                                      kWinRows, lane, guard);
-      }
-      if (!active || edge) {  // conv zero padding: rows outside [0, L)
-        __syncwarp();
-        for (int r = lane; r < G::kWarpRows; r += 32) {
-          const int t = q0 + r;
-          if (t < 0 || t >= P.L) *reinterpret_cast<uint4*>(yt + (size_t)r * 16) = make_uint4(0u, 0u, 0u, 0u);
-        }
-      }
-      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");  // image writes (generic) before the MMA reads (async)
-      __syncwarp();
-      if (lane == 0) {
-        mbar_arrive(xempty0 + 8 * xs);
-        mbar_arrive(fb);
-      }
-    }
-    guard.commit(P.status, 1);
-  }
-done:
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, 512);
-  }
-}
-
 // ------------------------------------------------------------------------------ layout helpers
 __global__ void to_chunked_bf16_kernel(const float* __restrict__ src, long long src_batch, long long src_c,
                                        long long src_t, __nv_bfloat16* __restrict__ dst, long long dst_batch,
@@ -1266,11 +1057,8 @@ extern "C" __attribute__((visibility("default"))) int64_t fh_tc_packed_weight_by
   return (int64_t)P * n_tiles * ((Cin + 15) / 16) * ntaps * bn * 32;
 }
 
-static int device_sms() { return fh::dev_sms(); }
-
-// Validates the arguments and derives the launch plan (tile shape, stages, shared-memory carve-up).  `budget_bytes` is
-// the shared memory the conv roles may use (0 = default).  Returns FH_OK (plain kernel), 1 (fused snake prologue) or < 0.
-static int tc_plan(const fh_tc_conv_args* a, void* stream, int budget_bytes, TcParams& p, int* smem_out) {
+// Validates the arguments and derives the launch plan (tile shape, stages, shared-memory carve-up).  Returns FH_OK or < 0.
+static int tc_plan(const fh_tc_conv_args* a, TcParams& p, int* smem_out) {
   FH_REQUIRE(a != nullptr, FH_ERR_BAD_SHAPE, "fh_tc_conv: null args");
   FH_REQUIRE(a->B > 0 && a->L > 0 && a->Cin > 0 && a->Cout > 0, FH_ERR_BAD_SHAPE, "fh_tc_conv: bad shape");
   FH_REQUIRE(a->Cin % 8 == 0, FH_ERR_BAD_SHAPE, "fh_tc_conv: Cin=%d must be a multiple of 8", a->Cin);
@@ -1310,38 +1098,21 @@ static int tc_plan(const fh_tc_conv_args* a, void* stream, int budget_bytes, TcP
   p.status = fh::status_word();
   p.B = a->B, p.L = a->L, p.Cin = a->Cin, p.Cout = a->Cout, p.ntaps = a->ntaps, p.P = a->P, p.bn = a->bn;
   p.n_tiles = (a->Cout + a->bn - 1) / a->bn;
-  const bool fused = a->x_f32 != nullptr;
   const bool two = a->two_cta != 0;
-  FH_REQUIRE(!(two && fused), FH_ERR_UNSUPPORTED_CFG, "fh_tc_conv: the CTA-pair kernel has no fused snake prologue");
   p.two_cta = two ? 1 : 0;
-  if (fused) {
-    FH_REQUIRE(a->P == 1 && p.n_tiles == 1 && a->bn <= 128 && a->Cin <= 128 && a->sn_a && a->sn_inv_b && a->sn_filt && !a->geglu,
-               FH_ERR_UNSUPPORTED_CFG, "fh_tc_conv: fused snake needs P == 1 and one N tile of <= 128 columns");
-    FH_REQUIRE(((uintptr_t)a->x_f32 % 16) == 0, FH_ERR_BAD_ALIGN, "fh_tc_conv: x_f32 must be 16-byte aligned");
-    FH_REQUIRE(!a->x_is_16 || a->fp16, FH_ERR_UNSUPPORTED_CFG, "fh_tc_conv: a 16-bit snake input must be fp16");
-    FH_REQUIRE(a->fp16, FH_ERR_UNSUPPORTED_CFG, "fh_tc_conv: the fused snake prologue produces fp16 operands");
-  }
   // sub-tiles: reuse each weight slot for up to 4 x 128 rows when the accumulators fit TMEM twice over
   int msub = 256 / a->bn;
   msub = msub >= 8 ? 8 : (msub >= 4 ? 4 : (msub >= 2 ? 2 : 1));  // 8 x 128 rows for bn <= 32 (24-channel last stage)
   // Wide tiles (bn > 128): the weight stream from L2 (bn*32 B per MMA) is the limiter, so two 128-row
   // sub-tiles share every weight slot even though the accumulators (2*bn columns) then fill TMEM and
   // the epilogue no longer overlaps the next tile -- worth it once a tile carries enough MMAs.
-  static int wide_msub = -1, wide_min = 96;
-  if (wide_msub < 0) {
-    const char* e = getenv("FH_TC_WIDE_MSUB");
-    wide_msub = e ? atoi(e) : 2;
-    const char* m = getenv("FH_TC_WIDE_MIN");
-    if (m) wide_min = atoi(m);
-  }
+  constexpr int kWideMsub = 2, kWideMinMmas = 96;
   // (Linear layers with many N tiles -- qkv, FF-in: 64 MMAs per tile -- gain 10 % from the shared weight slot as well;
   // the 4-tile output projection loses 15 % and keeps one sub-tile)
   const long long mmas_per_sub = (long long)a->ntaps * ((a->Cin + 15) / 16);
-  if (a->bn > 128 && wide_msub == 2 && (mmas_per_sub >= wide_min || (mmas_per_sub >= 64 && p.n_tiles >= 8))) msub = 2;
-  while (!fused && msub > 1 &&
-         (long long)a->B * a->P * ((a->L + 128 * msub - 1) / (128 * msub)) * p.n_tiles < 2 * 148)
+  if (a->bn > 128 && (mmas_per_sub >= kWideMinMmas || (mmas_per_sub >= 64 && p.n_tiles >= 8))) msub = kWideMsub;
+  while (msub > 1 && (long long)a->B * a->P * ((a->L + 128 * msub - 1) / (128 * msub)) * p.n_tiles < 2 * 148)
     msub >>= 1;
-  // (fused: snake work units are 128 window rows = one sub-tile, any msub works)
   p.msub = msub;
   p.acc_stages = (2 * msub * a->bn <= 512) ? 2 : 1;
   p.m_stride = p.m_valid = 128 * msub;
@@ -1368,53 +1139,26 @@ static int tc_plan(const fh_tc_conv_args* a, void* stream, int budget_bytes, TcP
   }
   FH_REQUIRE(span <= kMaxSpan, FH_ERR_UNSUPPORTED_CFG, "fh_tc_conv: tap span %d exceeds %d rows", span, kMaxSpan);
   p.tap_arith = arith;
-  {
-    static int tap_pair_on = -1;
-    if (tap_pair_on < 0) {
-      const char* e = getenv("FH_TC_TAP_PAIR");
-      tap_pair_on = e ? atoi(e) : 1;
-    }
-    p.tap_pair = (tap_pair_on && p.ci_odd && arith && a->P == 1 && a->ntaps >= 2 && p.tap_step[0] > 0 && !fused && !two) ? 1 : 0;
-  }
-  if (fused) {  // aligned A window of exactly 128 msub rows: a tile keeps 128 msub - span output rows
-    p.m_stride = p.m_valid = 128 * msub - span;
-    p.m_tiles = (a->L + p.m_stride - 1) / p.m_stride;
-  }
+  p.tap_pair = (p.ci_odd && arith && a->P == 1 && a->ntaps >= 2 && p.tap_step[0] > 0 && !two) ? 1 : 0;
   if (two) p.m_tiles = (p.m_tiles + 1) / 2;  // CTA PAIRS along M (decode_tile); an odd tail leaves one void tile
   const long long total = (long long)p.B * p.P * p.m_tiles * p.n_tiles * (two ? 2 : 1);
   FH_REQUIRE(total < (1ll << 31), FH_ERR_BAD_SHAPE, "fh_tc_conv: too many tiles");
   p.total_tiles = (int)total;
   {
-    static int use_v8 = -1;
-    if (use_v8 < 0) {
-      const char* e = getenv("FH_TC_V8");
-      use_v8 = e ? atoi(e) : 1;
-    }
     const bool out_ok = a->out_is_16 || (((uintptr_t)a->out % 32) == 0 && a->out_batch % 8 == 0 && a->out_chunk % 8 == 0 &&
                                          a->out_row % 8 == 0);
     const bool res_ok = a->res == nullptr || a->res_is_16 ||
                         (((uintptr_t)a->res % 32) == 0 && a->res_batch % 8 == 0 && a->res_chunk % 8 == 0 && a->res_row % 8 == 0);
     const bool acc_ok = !(a->accumulate && a->acc_src) ||
                         (((uintptr_t)a->acc_src % 32) == 0 && a->out_batch % 8 == 0 && a->out_chunk % 8 == 0 && a->out_row % 8 == 0);
-    p.v8 = (use_v8 && out_ok && res_ok && acc_ok) ? 1 : 0;
+    p.v8 = (out_ok && res_ok && acc_ok) ? 1 : 0;
   }
   p.wrows = 128 * msub + span;
   p.arows_pad = 128 * msub + kMaxSpan;
-  if (fused) {
-    p.rows_per_chunk = (int)(a->a_chunk / 8);
-    p.xf = a->x_f32, p.sn_a = a->sn_a, p.sn_ib = a->sn_inv_b, p.sn_filt = a->sn_filt;
-  }
-  // taps per stage: a weight slot of <= 32 KB (<= 48 KB for narrow tiles, so that all taps of a ci-pair share
-  // one activation window fetch), with the taps spread evenly over the groups (11 taps -> 6+5, not 10+1)
-  static int slot_small_kb = 0, slot_wide_kb = 0;
-  if (!slot_small_kb) {
-    const char* e1 = getenv("FH_TC_SLOT_SMALL_KB");
-    const char* e2 = getenv("FH_TC_SLOT_WIDE_KB");
-    slot_small_kb = e1 ? atoi(e1) : 48;
-    slot_wide_kb = e2 ? atoi(e2) : 48;
-  }
-  int tg = ((a->bn <= 128 ? slot_small_kb : slot_wide_kb) * 1024) / (a->bn * 32);
-  if (fused) tg = a->ntaps;  // one stage = one ci-pair with all its taps
+  // taps per stage: a weight slot of <= 48 KB for narrow and wide tiles alike (for narrow tiles all taps of a ci-pair
+  // then share one activation window fetch), with the taps spread evenly over the groups (11 taps -> 6+5, not 10+1)
+  constexpr int kSlotBytes = 48 * 1024;
+  int tg = kSlotBytes / (a->bn * 32);
   if (tg < 1) tg = 1;
   if (tg > a->ntaps) tg = a->ntaps;
   p.n_groups = (a->ntaps + tg - 1) / tg;
@@ -1422,121 +1166,46 @@ static int tc_plan(const fh_tc_conv_args* a, void* stream, int budget_bytes, TcP
   p.tg = tg;
   // ci-pairs per stage: a stage should carry >= ~12 MMAs so that its barrier round trip is amortised (Linear layers are
   // one tap per ci-pair, k = 3 convs three), as long as at least 3-4 stages still fit
-  static int kc_target = -1;
-  if (kc_target < 0) {
-    const char* e = getenv("FH_TC_KC_MMAS");
-    kc_target = e ? atoi(e) : 12;
-  }
-  static int kc_target2 = -1;  // CTA pairs: a stage costs two barrier round trips more (relay, multicast commit)
-  if (kc_target2 < 0) {
-    const char* e = getenv("FH_TC_KC_MMAS2");
-    kc_target2 = e ? atoi(e) : 24;
-  }
+  constexpr int kKcMmas = 12;
+  constexpr int kKcMmas2 = 24;  // CTA pairs: a stage costs two barrier round trips more (relay, multicast commit)
+  constexpr int kSmemBudget = 200 * 1024;  // shared memory of the stages and the bias table without a residual ring
   int kc = 1;
-  if (!fused && p.n_groups == 1 && kc_target > 0) {
+  if (p.n_groups == 1) {
     const int pair_bytes = 2 * p.arows_pad * 16 + a->ntaps * (two ? a->bn / 2 : a->bn) * 32;
-    const int kct = two ? kc_target2 : kc_target;
+    const int kct = two ? kKcMmas2 : kKcMmas;
     kc = (kct + a->ntaps * msub - 1) / (a->ntaps * msub);
     if (kc > 4) kc = 4;
     if (kc > p.ci_pairs) kc = p.ci_pairs;
-    while (kc > 1 && (200 * 1024 - 1024 - 8192) / (kc * pair_bytes) < 4) --kc;
+    while (kc > 1 && (kSmemBudget - 1024 - 8192) / (kc * pair_bytes) < 4) --kc;
   }
   p.kc = kc;
   p.stage_bytes = kc * (2 * p.arows_pad * 16 + tg * (two ? a->bn / 2 : a->bn) * 32);  // a CTA of a pair holds half of every weight slot
   p.stage_bytes = (p.stage_bytes + 127) & ~127;
-  static int budget_kb = 0;
-  if (!budget_kb) {
-    const char* e = getenv("FH_TC_SMEM_KB");
-    budget_kb = e ? atoi(e) : 200;
-    if (budget_kb < 64 || budget_kb > 220) budget_kb = 200;
-  }
-  const int budget = budget_bytes > 0 ? budget_bytes : budget_kb * 1024;
-  static int fast_on = -1;
-  if (fast_on < 0) {
-    const char* e = getenv("FH_TC_FAST_EPI");
-    fast_on = e ? atoi(e) : 1;
-  }
   const int bias_tab = a->bias ? ((p.n_tiles * a->bn + 15) & ~15) * 4 : 64;
-  p.fast_epi = (fast_on && p.v8 && !a->geglu && !p.act_gelu && !(a->res && a->res_is_16) && bias_tab <= 8192 &&
+  p.fast_epi = (p.v8 && !a->geglu && !p.act_gelu && !(a->res && a->res_is_16) && bias_tab <= 8192 &&
                 (!a->out_is_16 || (a->res == nullptr && !a->accumulate) || (a->accumulate && a->acc_src && a->res))) ? 1 : 0;
   FH_REQUIRE(p.fast_epi || !(a->accumulate && a->out_is_16), FH_ERR_UNSUPPORTED_CFG,
              "fh_tc_conv: accumulate into a 16-bit output is only implemented by the specialised epilogue");
   const int tail = p.fast_epi ? bias_tab : 0;
-  if (fused) {
-    // this kernel owns the SM: conv stages (3-4: the eight snake warps spread over up to four of them), then the x ring
-    // (one slot per 272-row unit window, at least one per snake warp)
-    const int fbudget = 222 * 1024;
-    const int grid_hint = p.total_tiles < device_sms() ? p.total_tiles : device_sms();
-    static int pro_nb = 0, pro_st = -1;
-    if (!pro_nb) {
-      const char* e = getenv("FH_PRO_NB");
-      pro_nb = (e && atoi(e) == 16) ? 16 : 8;
-      const char* e2 = getenv("FH_PRO_STAGES");
-      pro_st = e2 ? atoi(e2) : 0;
-    }
-    const int kProNB = (pro_nb == 16 && msub >= 2) ? 16 : 8;
-    p.pro_nb = kProNB;
-    p.xs_bytes = (16 * kProNB + 16) * (a->x_is_16 ? 16 : 32);
-    // ncu (profiles/r2_ncu_fused_*.txt): with one window slot per snake warp a third of the snake warps' samples sat on
-    // the window barrier -- the DRAM latency of every unit was exposed.  Two to three slots per warp hide it; the conv
-    // stages only need to hold the >= 8 units the eight warps work on, plus one stage for the MMAs in flight.
-    const int units_per_stage = 2 * (128 * msub) / (16 * kProNB);
-    int st = units_per_stage >= 8 ? 2 : 3;
-    if (pro_st >= 2 && pro_st <= 4) st = pro_st;
-    while (st > 2 && 1024 + st * p.stage_bytes + tail + 16 * p.xs_bytes + 16 * kProXMax > fbudget) --st;
-    const int room = fbudget - 1024 - st * p.stage_bytes - tail - 16 * kProXMax - 128;
-    int xd = room / p.xs_bytes;
-    if (xd > kProXMax) xd = kProXMax;
-    // >= 8 x slots: the consumer of window n has finished window n - 8 itself, so it can never be two fills ahead of the
-    // producer on a slot (mbarrier parity waits cannot tell generation g from g - 2)
-    // Active snake warps W: a warp has consumed window n - W itself before it waits for window n, so every parity wait is
-    // unambiguous as long as the x ring has >= W slots and the 8 stage barriers cover >= W units.
-    {
-      const int upc = (128 * msub) / (16 * kProNB);                // units per chunk and tile
-      const int min_units = p.ci_odd ? upc : 2 * upc;              // real units of the smallest stage
-      int w = kProSnakeWarps;
-      if (w > kMaxStages * min_units) w = kMaxStages * min_units;
-      if (w > xd) w = xd;
-      p.snake_warps = w;
-    }
-    FH_REQUIRE(xd >= 4 && p.snake_warps >= 1, FH_ERR_UNSUPPORTED_CFG, "fh_tc_conv: fused snake stages (%d bytes each) do not fit shared memory",
-               p.stage_bytes);
-    FH_REQUIRE(((long long)p.total_tiles / grid_hint + 2) * p.ci_pairs * 16 < (1ll << 30), FH_ERR_BAD_SHAPE,
-               "fh_tc_conv: too many fused-snake units per CTA");
-    p.stages = st;
-    p.empty_ring = kMaxStages;
-    p.x_stages = xd;
-    p.xs_off = (1024 + st * p.stage_bytes + tail + 127) & ~127;
-    p.err_flag = fh::err_word();
-    *smem_out = p.xs_off + xd * p.xs_bytes + 16 * kProXMax;
-    return 1;
-  }
   // residual rows through the cp.async ring (epilogue_fast<.., RES_ASYNC>): the HBM-bound launches (<= 96 output channels in
   // one N tile, fp32 residual rows of 8 floats, P == 1) whose residual stream was latency-bound; the ring (64 KB) comes
   // out of the stage budget, which these launches do not need (a tile is 2 - 6 stages)
-  static int res_async_on = -1, ew_max_bn = -1, ew16_mmas = 64;
-  if (res_async_on < 0) {
-    const char* e = getenv("FH_TC_RES_ASYNC");
-    res_async_on = e ? atoi(e) : 1;
-    const char* w = getenv("FH_TC_EW_BN");  // widest N tile that runs with more than eight epilogue warps (0 = never)
-    ew_max_bn = w ? atoi(w) : 96;
-    const char* n = getenv("FH_TC_EW16_MMAS");  // sixteen epilogue warps up to this many MMAs per tile, twelve above
-    if (n) ew16_mmas = atoi(n);
-  }
-  const int res_async_max = res_async_on > 1 ? res_async_on : 192;
+  constexpr int kResAsyncMaxCout = 192;
+  constexpr int kEpiWideMaxBn = 96;  // widest N tile that runs with more than eight epilogue warps
+  constexpr int kEw16Mmas = 64;      // sixteen epilogue warps up to this many MMAs per tile, twelve above
   // Epilogue warps.  The narrow (HBM-bound) shapes were paced by their eight epilogue warps: two per scheduler, each
   // issuing once every ~5 cycles (fixed-latency dependencies), so more warps are more throughput -- sixteen reach the
   // HBM roofline on the k = 3 shapes.  With many MMAs per tile (k >= 7) sixteen starve the single MMA-issuing warp of
   // issue slots on its scheduler (measured 20 - 30 % slower than twelve), so those run with twelve.
   p.epi_warps = 8;
-  if (p.fast_epi && !two && a->bn <= ew_max_bn && budget_bytes == 0)
-    p.epi_warps = (a->ntaps * p.ci_pairs * p.msub <= ew16_mmas) ? 16 : 12;
+  if (p.fast_epi && !two && a->bn <= kEpiWideMaxBn)
+    p.epi_warps = (a->ntaps * p.ci_pairs * p.msub <= kEw16Mmas) ? 16 : 12;
   int ring = 0;
-  if (res_async_on && p.fast_epi && !two && a->res != nullptr && !a->res_is_16 && a->P == 1 && a->res_row == 8 &&
-      a->Cout <= res_async_max && p.msub * (a->bn >> 4) >= (p.epi_warps + 3) / 4 && budget_bytes == 0 &&
+  if (p.fast_epi && !two && a->res != nullptr && !a->res_is_16 && a->P == 1 && a->res_row == 8 &&
+      a->Cout <= kResAsyncMaxCout && p.msub * (a->bn >> 4) >= (p.epi_warps + 3) / 4 &&
       (216 * 1024 - 1024 - tail - 128 - res_ring_bytes(p.epi_warps)) / p.stage_bytes >= 2)
     ring = res_ring_bytes(p.epi_warps);
-  int stages = ((ring ? 216 * 1024 - 128 - ring : budget) - 1024 - tail) / p.stage_bytes;
+  int stages = ((ring ? 216 * 1024 - 128 - ring : kSmemBudget) - 1024 - tail) / p.stage_bytes;
   if (stages > kMaxStages) stages = kMaxStages;
   FH_REQUIRE(stages >= 2, FH_ERR_UNSUPPORTED_CFG, "fh_tc_conv: stage of %d bytes does not fit twice", p.stage_bytes);
   p.stages = stages;
@@ -1551,24 +1220,10 @@ static int tc_plan(const fh_tc_conv_args* a, void* stream, int budget_bytes, TcP
 extern "C" __attribute__((visibility("default"))) int fh_tc_conv(const fh_tc_conv_args* a, void* stream) {
   TcParams p;
   int smem = 0;
-  const int rc = tc_plan(a, stream, 0, p, &smem);
-  if (rc != FH_OK && rc != 1) return rc;
-  const int num_sms = device_sms();
+  const int rc = tc_plan(a, p, &smem);
+  if (rc != FH_OK) return rc;
+  const int num_sms = fh::dev_sms();
   const int grid = p.total_tiles < num_sms ? p.total_tiles : num_sms;
-  if (rc == 1) {  // fused snake prologue
-    static int set_a[64] = {0}, set_b[64] = {0}, set_c[64] = {0}, set_d[64] = {0};
-    cudaError_t e;
-#define FH_PRO_LAUNCH(IN16, NB, TAB)                                                              \
-  e = fh::ensure_dyn_smem(tc_conv_snakepro_kernel<IN16, NB>, smem, TAB);                          \
-  FH_REQUIRE(e == cudaSuccess, FH_ERR_CUDA, "fh_tc_conv: cannot opt in to %d bytes of smem: %s", smem, cudaGetErrorString(e)); \
-  tc_conv_snakepro_kernel<IN16, NB><<<grid, kProThreads, smem, (cudaStream_t)stream>>>(p)
-    if (a->x_is_16 && p.pro_nb == 16) { FH_PRO_LAUNCH(true, 16, set_a); }
-    else if (a->x_is_16) { FH_PRO_LAUNCH(true, 8, set_b); }
-    else if (p.pro_nb == 16) { FH_PRO_LAUNCH(false, 16, set_c); }
-    else { FH_PRO_LAUNCH(false, 8, set_d); }
-#undef FH_PRO_LAUNCH
-    return fh::check_launch("fh_tc_conv(fused snake)");
-  }
   if (p.two_cta) {
     static int smem_set2[64] = {0};
     cudaError_t e = fh::ensure_dyn_smem(tc_conv2_kernel, smem, smem_set2);

@@ -2,7 +2,6 @@
 // fh_tc_conv consumes: fused anti-aliased Snake/SnakeBeta (alias_free_torch/act.py:23-28,
 // resample.py:25-33, filter.py:86-94, activations.py:48-59,107-119) and conv_post + tanh
 // (bigvgan/models.py:189-192).  The residual stream stays fp32; only MMA operands are 16-bit.
-#include <stdlib.h>
 #include "common.cuh"
 #include "snake_worker.cuh"
 #include "snake_mma.cuh"
@@ -10,8 +9,7 @@
 namespace {
 
 // ------------------------------------------------------------------------------ anti-aliased snake
-// The kernel body lives in snake_worker.cuh (shared with the dual conv + snake kernel of tc_conv.cu): persistent CTAs
-// of one 128-thread worker each, 17 outputs per thread.
+// The kernel body lives in snake_worker.cuh: persistent CTAs of one 128-thread worker each, 17 outputs per thread.
 constexpr int PR = 17;
 
 template <int OUT_KIND, bool BULK_OUT>
@@ -20,25 +18,23 @@ __global__ void __launch_bounds__(128, 4) snake_aa_chunked_tma_kernel(const __gr
   fh::snake_worker<OUT_KIND, BULK_OUT, PR>(S, snake_smem, threadIdx.x, blockIdx.x, gridDim.x, 0);
 }
 
-// fp16 output mode: both FIR filters as Toeplitz MMAs (snake_mma.cuh).  MODE bit 0: hi/lo split of the input,
-// bit 1: hi/lo split of the filter taps.
-template <int MODE, int NB, int MINB, bool IN16, bool SPLIT_OUT, int WBUF>
+// fp16 output mode: both FIR filters as Toeplitz MMAs (snake_mma.cuh).  SPLIT_X: hi/lo split of the input.
+template <bool SPLIT_X, int NB, int MINB, bool IN16, bool SPLIT_OUT>
 __global__ void __launch_bounds__(128, MINB) snake_aa_mma_kernel(const __grid_constant__ fh::SnakeParams S) {
   extern __shared__ __align__(128) unsigned char snake_smem[];
-  fh::snake_mma_cta<(MODE & 1) != 0, (MODE & 2) != 0, NB, IN16, SPLIT_OUT, WBUF>(S, snake_smem, threadIdx.x, blockIdx.x,
-                                                                                 gridDim.x);
+  fh::snake_mma_cta<SPLIT_X, NB, IN16, SPLIT_OUT>(S, snake_smem, threadIdx.x, blockIdx.x, gridDim.x);
 }
 
-template <int MODE, int NB, int MINB, bool IN16 = false, bool SPLIT_OUT = false, int WBUF = 2>
+template <bool SPLIT_X, int NB, int MINB, bool IN16 = false, bool SPLIT_OUT = false>
 void launch_snake_mma(fh::SnakeParams sp, int B, int C, int L, int sms, cudaStream_t stream) {
   using G = fh::SnakeMmaGeom<NB>;
   static int smem_set[64] = {0};
-  fh::ensure_dyn_smem(snake_aa_mma_kernel<MODE, NB, MINB, IN16, SPLIT_OUT, WBUF>, G::smem_bytes(IN16, SPLIT_OUT, WBUF), smem_set);
+  fh::ensure_dyn_smem(snake_aa_mma_kernel<SPLIT_X, NB, MINB, IN16, SPLIT_OUT>, G::smem_bytes(IN16, SPLIT_OUT), smem_set);
   sp.ntile = (L + G::kRows - 1) / G::kRows;
   const long long total = (long long)sp.ntile * (C / 8) * B;
   sp.total = (int)total;
   const int grid = (int)(total < (long long)sms * MINB ? total : (long long)sms * MINB);
-  snake_aa_mma_kernel<MODE, NB, MINB, IN16, SPLIT_OUT, WBUF><<<grid, 128, G::smem_bytes(IN16, SPLIT_OUT, WBUF), stream>>>(sp);
+  snake_aa_mma_kernel<SPLIT_X, NB, MINB, IN16, SPLIT_OUT><<<grid, 128, G::smem_bytes(IN16, SPLIT_OUT), stream>>>(sp);
 }
 
 // conv_post (C -> 1, k = 7, zero padding) + tanh on the chunked fp32 layout (bigvgan/models.py:190-192).  HBM-bound:
@@ -235,30 +231,17 @@ extern "C" __attribute__((visibility("default"))) int fh_snake_aa_chunked(
   FH_REQUIRE(out_kind >= 0 && out_kind <= 2, FH_ERR_BAD_SHAPE, "fh_snake_aa_chunked: out_kind must be 0 (fp32), 1 (bf16), 2 (fp16)");
   FH_REQUIRE(((uintptr_t)x % 16) == 0 && (batch_stride % 8) == 0 && (chunk_stride % 8) == 0, FH_ERR_BAD_ALIGN,
              "fh_snake_aa_chunked: x must be 16-byte aligned and strides multiples of 8");
-  static int mma_mode = -2;  // FH_SNAKE_MMA: -1 = scalar kernel, 0..3 = Toeplitz-MMA kernel (bit 0 split x, bit 1 split taps)
-  if (mma_mode == -2) {
-    const char* e = getenv("FH_SNAKE_MMA");
-    mma_mode = e ? atoi(e) : 0;  // the input split buys < 0.3 dB of end-to-end SNR for 15 % more kernel time
-    if (mma_mode < -1 || mma_mode > 3) mma_mode = 0;
-  }
-  const bool use_mma = out_kind == 2 && mma_mode >= 0 && row0 >= fh::SnakeMmaGeom<8>::kHalo;
+  // fp16 output: the Toeplitz-MMA kernel.  Its hi/lo split of the input (as in fh_snake_aa_chunked_split) buys < 0.3 dB
+  // of end-to-end SNR for 15 % more kernel time; neither it nor the hi/lo split of the filter taps was ever the default,
+  // and both were removed.  A left halo shorter than the MMA kernel's window falls back to the scalar kernel.
+  const bool use_mma = out_kind == 2 && row0 >= fh::SnakeMmaGeom<8>::kHalo;
   constexpr int kTileRows = fh::SnakeGeom<PR>::kRows;
   const int ntile = (L + kTileRows - 1) / kTileRows;
   const long long total = (long long)ntile * (C / 8) * B;
   FH_REQUIRE(total <= 2147483647LL && row0 >= 5, FH_ERR_BAD_SHAPE, "fh_snake_aa_chunked: needs a left halo of >= 5 rows");
   const int sms = fh::dev_sms();
-  static int per_sm = 0;  // persistent CTAs per SM (4 fill the SM)
-  if (!per_sm) {
-    const char* e = getenv("FH_SNAKE_CTAS_PER_SM");
-    per_sm = e ? atoi(e) : 4;
-    if (per_sm < 1 || per_sm > 4) per_sm = 4;
-  }
-  const int grid = (int)(total < (long long)sms * per_sm ? total : (long long)sms * per_sm);
-  static int bulk = -1;
-  if (bulk < 0) {
-    const char* e = getenv("FH_SNAKE_BULK");
-    bulk = e ? atoi(e) : 1;
-  }
+  constexpr int kPerSm = 4;  // persistent CTAs per SM of the scalar kernel (4 fill the SM)
+  const int grid = (int)(total < (long long)sms * kPerSm ? total : (long long)sms * kPerSm);
   fh::SnakeParams sp;
   sp.x = x, sp.y = y, sp.a = a, sp.inv_b = inv_b, sp.filt = filt;
   sp.batch_stride = batch_stride, sp.chunk_stride = chunk_stride, sp.y_batch_stride = batch_stride, sp.lo_offset = 0;
@@ -266,34 +249,19 @@ extern "C" __attribute__((visibility("default"))) int fh_snake_aa_chunked(
   sp.status = fh::status_word();
   if (use_mma) {
     FH_REQUIRE((long long)((L + 511) / 512) * (C / 8) * B <= 2147483647LL, FH_ERR_BAD_SHAPE, "fh_snake_aa_chunked: too many work items");
-    cudaStream_t cs = (cudaStream_t)stream;
     // 8 blocks of 8 outputs per half-segment, 4 CTAs per SM (4-block segments at 6 CTAs per SM: 142 vs 118 ms per step)
-    // 128-output segments at 2 CTAs per SM (default) against 64-output segments at 4: 6 % less halo work (MUFU, MMAs)
-    // and half the warps -- 87.0 vs 93.3 ms per step; FH_SNAKE_NB=8 selects the smaller tiles
-    static int nb16 = -1;
-    if (nb16 < 0) {
-      const char* e = getenv("FH_SNAKE_NB");
-      nb16 = (e && atoi(e) == 8) ? 0 : 1;
-    }
-    static int wbuf1 = -1;  // FH_SNAKE_WBUF=1: single input window, 3 CTAs (12 warps) per SM instead of 2
-    if (wbuf1 < 0) {
-      const char* e = getenv("FH_SNAKE_WBUF");
-      wbuf1 = (e && atoi(e) == 1) ? 1 : 0;
-    }
-    if (mma_mode == 0 && nb16 && wbuf1) launch_snake_mma<0, 16, 3, false, false, 1>(sp, B, C, L, sms, cs);
-    else if (mma_mode == 0 && nb16) launch_snake_mma<0, 16, 2>(sp, B, C, L, sms, cs);
-    else if (mma_mode == 0) launch_snake_mma<0, 8, 4>(sp, B, C, L, sms, cs);
-    else if (mma_mode == 3) launch_snake_mma<3, 8, 4>(sp, B, C, L, sms, cs);
-    else launch_snake_mma<1, 8, 4>(sp, B, C, L, sms, cs);
+    // 128-output segments at 2 CTAs per SM against 64-output segments at 4: 6 % less halo work (MUFU, MMAs)
+    // and half the warps -- 87.0 vs 93.3 ms per step.  A single input window per CTA (3 CTAs per SM) measured no better
+    // and was removed.
+    launch_snake_mma<false, 16, 2>(sp, B, C, L, sms, (cudaStream_t)stream);
     return fh::check_launch("fh_snake_aa_chunked");
   }
+  // scalar kernel; 16-bit outputs go to HBM through a bulk store of the output tile
   constexpr int kSmem = fh::SnakeGeom<PR>::kSmemBytes;
 #define FH_SNAKE_LAUNCH(KIND, BULK) snake_aa_chunked_tma_kernel<KIND, BULK><<<grid, 128, kSmem, (cudaStream_t)stream>>>(sp)
   if (out_kind == 0) FH_SNAKE_LAUNCH(0, false);
-  else if (out_kind == 1 && bulk) FH_SNAKE_LAUNCH(1, true);
-  else if (out_kind == 1) FH_SNAKE_LAUNCH(1, false);
-  else if (bulk) FH_SNAKE_LAUNCH(2, true);
-  else FH_SNAKE_LAUNCH(2, false);
+  else if (out_kind == 1) FH_SNAKE_LAUNCH(1, true);
+  else FH_SNAKE_LAUNCH(2, true);
 #undef FH_SNAKE_LAUNCH
   return fh::check_launch("fh_snake_aa_chunked");
 }
@@ -317,7 +285,7 @@ extern "C" __attribute__((visibility("default"))) int fh_snake_aa_chunked_split(
   sp.lo_offset = (int64_t)(C / 8) * chunk_stride;
   sp.row0 = row0, sp.nchunk = C / 8, sp.L = L, sp.ntile = 0, sp.total = 0, sp.fp16 = 1;
   sp.status = fh::status_word();
-  launch_snake_mma<1, 8, 3, false, true>(sp, B, C, L, fh::dev_sms(), (cudaStream_t)stream);
+  launch_snake_mma<true, 8, 3, false, true>(sp, B, C, L, fh::dev_sms(), (cudaStream_t)stream);
   return fh::check_launch("fh_snake_aa_chunked_split");
 }
 
@@ -338,27 +306,10 @@ extern "C" __attribute__((visibility("default"))) int fh_snake_aa_chunked_h(
   sp.batch_stride = batch_stride, sp.chunk_stride = chunk_stride, sp.y_batch_stride = batch_stride, sp.lo_offset = 0;
   sp.row0 = row0, sp.nchunk = C / 8, sp.L = L, sp.ntile = 0, sp.total = 0, sp.fp16 = 1;
   sp.status = fh::status_word();
-  // FH_SNAKE_H_CTAS=5: five CTAs per SM fit with the half-size fp16 windows (33 KB, 90 registers) -- measured SLOWER
-  // (101.5 vs 98.3 ms per step, like every other occupancy increase of this kernel: it is not latency-bound)
-  static int per_sm = 0;
-  if (!per_sm) {
-    const char* e = getenv("FH_SNAKE_H_CTAS");
-    per_sm = e ? atoi(e) : 4;
-  }
-  static int nb16 = -1;
-  if (nb16 < 0) {
-    const char* e = getenv("FH_SNAKE_NB");
-    nb16 = (e && atoi(e) == 8) ? 0 : 1;
-  }
-  static int wbuf1 = -1;  // FH_SNAKE_WBUF=1: single input window, 4 CTAs (16 warps) per SM instead of 3
-  if (wbuf1 < 0) {
-    const char* e = getenv("FH_SNAKE_WBUF");
-    wbuf1 = (e && atoi(e) == 1) ? 1 : 0;
-  }
-  if (nb16 && wbuf1) launch_snake_mma<0, 16, 4, true, false, 1>(sp, B, C, L, sms, (cudaStream_t)stream);
-  else if (nb16) launch_snake_mma<0, 16, 3, true>(sp, B, C, L, sms, (cudaStream_t)stream);
-  else if (per_sm == 5) launch_snake_mma<0, 8, 5, true>(sp, B, C, L, sms, (cudaStream_t)stream);
-  else launch_snake_mma<0, 8, 4, true>(sp, B, C, L, sms, (cudaStream_t)stream);
+  // 128-output segments at 3 CTAs per SM.  Five CTAs per SM fit with 64-output segments and the half-size fp16 windows
+  // (33 KB, 90 registers) -- measured SLOWER (101.5 vs 98.3 ms per step, like every other occupancy increase of this
+  // kernel: it is not latency-bound); a single input window per CTA (4 CTAs per SM) measured no better.  Both were removed.
+  launch_snake_mma<false, 16, 3, true>(sp, B, C, L, sms, (cudaStream_t)stream);
   return fh::check_launch("fh_snake_aa_chunked_h");
 }
 

@@ -77,30 +77,16 @@ class Engine:
         self._touch_log = None         # {id: object} while a CUDA graph is warmed up / captured: what the graph must keep alive
         self.profile = None
         import os as _os
-        self.voc_streams = int(_os.environ.get("FH_VOC_STREAMS", "1"))
         self.tc_attention = _os.environ.get("FH_TC_ATTENTION", "1") != "0"  # tensor-core split-operand attention
         self._cool_ms = float(_os.environ.get("FH_PROFILE_COOL_MS", "0"))
         self.attn5 = _os.environ.get("FH_ATTN_TC5", "1") != "0"  # tcgen05 / TMEM kernel (0: the mma.sync kernel)
-        # fp16 path, stages of <= 128 channels: FH_FUSE_SNAKE=1 runs the anti-aliased snake INSIDE the conv kernel as the
-        # producer of its A operand (tc_conv_snakepro_kernel: 16 instead of 24 HBM bytes per element of an AMP unit).
-        # Parity-tested, but measured at the same step time as the separate launches on B200 (311-319 vs 312 ms; ncu in
-        # profiles/r2_ncu_fused_snake_conv.txt: the snake warps, not HBM, pace the kernel), so the separate launches
-        # stay the default.
-        self.fuse_snake = self.fp16 == 1 and not self.split and _os.environ.get("FH_FUSE_SNAKE", "0") != "0"
-        # CTA-pair kernel (tc_conv2_kernel: cta_group::2 MMA, M = 256, one weight stream per SM pair).  Decided per layer
-        # at load time because the packed weight layout differs.  FH_TC_2CTA: "auto" (default) = the shapes it wins on
-        # (_pair_wins, measured per shape on B200), "1" = every tcgen05 convolution / Linear, "0" = never.
-        self.two_cta_mode = _os.environ.get("FH_TC_2CTA", "auto") if (self.tc and not self.fuse_snake) else "0"
-        self.two_cta = self.two_cta_mode == "1"
         # fp16 path: the first convolution of an AMP unit writes fp16 rows and the snake behind it reads them as MMA
         # operands (fh_snake_aa_chunked_h) -- the fp32 round trip of that tensor disappears
-        self.y16 = self.fp16 and not self.split and _os.environ.get("FH_Y16", "1") != "0"
+        self.y16 = self.fp16 and not self.split
         # AMP branches of a stage on parallel streams for small batches (B = 1 latency path)
-        self.branch_streams = _os.environ.get("FH_BRANCH_STREAMS", "1") != "0"
+        self.branch_streams = True
         self.branch_streams_max_batch = 4
         self._branch_streams = []
-        self.pp_fused = _os.environ.get("FH_PP_FUSED", "1") != "0"  # spectrogram-free post-processing
-        self._side_streams = []
         self._time_cache: "collections.OrderedDict[float, dict]" = collections.OrderedDict()  # LRU, <= 512 grid values
         dev = self.device
         with torch.cuda.device(dev):
@@ -262,19 +248,17 @@ class Engine:
         profiles/r2_pair_vs_single.txt): 192 / 384 output channels with >= 7 taps gain 14-25 % (their weight stream per SM
         halves), the 96-channel k = 11 first convolutions 17 %; HBM-bound residual launches, k = 3 shapes, the upsamplers
         and the Linear layers lose 3-20 % to the two extra barrier hops per stage; 768 channels are at the tensor peak
-        either way."""
-        if self.two_cta_mode != "auto":
-            return self.two_cta_mode == "1"
+        either way.  Decided per layer at load time because the packed weight layout differs."""
         if P != 1:
             return False
         if 192 <= cout <= 384 and ntaps >= 7:
             return True
         return cout == 96 and ntaps >= 11 and not residual
 
-    def _mk_tc(self, tconv: packing.TappedConv, cin_pad=None, cout_pad=None, bn=None, split=False, two_cta=None) -> _TcWeight:
+    def _mk_tc(self, tconv: packing.TappedConv, cin_pad=None, cout_pad=None, bn=None, split=False, two_cta=False) -> _TcWeight:
         r = _TcWeight()
         cin_alg = tconv.cin
-        r.two_cta = self.two_cta if two_cta is None else bool(two_cta)
+        r.two_cta = bool(two_cta)
         if split:  # hi + lo activation operand: doubled input channels, duplicated weights
             cin_pad = cin_pad or packing.round_up(tconv.cin, 8)
             tconv = packing.split_input(tconv, cin_pad)
@@ -343,7 +327,7 @@ class Engine:
         filt_up = sd[prefix + "upsample.filter"].flatten()
         filt_dn = sd[prefix + "downsample.lowpass.filter"].flatten()
         if not torch.equal(filt_up, filt_dn):
-            raise ValueError("up/down anti-alias filters differ; the fused snake kernel expects one 12-tap filter")
+            raise ValueError("up/down anti-alias filters differ; the snake kernels expect one 12-tap filter")
         return a, ib, filt_up.contiguous()
 
     def _prep_vocoder(self):
@@ -478,14 +462,9 @@ class Engine:
         return out
 
     def _tc_conv(self, rec: _TcWeight, a, a_batch, a_chunk, a_row0, out, out_strides, out_bf16, B, L, res=None,
-                 res_strides=(0, 0, 0), res_bf16=0, alpha=1.0, beta=0.0, accumulate=0, geglu=0, xf=None, snake=None, act=0,
-                 acc_src=None, x16=False):
+                 res_strides=(0, 0, 0), res_bf16=0, alpha=1.0, beta=0.0, accumulate=0, geglu=0, act=0, acc_src=None):
         args = _lib.TcConvArgs()
         args.a, args.a_batch, args.a_chunk, args.a_row0 = _ptr(a), a_batch, a_chunk, a_row0
-        if xf is not None:  # fused anti-aliased snake prologue: A = Activation1d(xf), computed in the kernel
-            args.x_f32 = xf.data_ptr()
-            args.x_is_16 = 1 if x16 else 0
-            args.sn_a, args.sn_inv_b, args.sn_filt = snake[0].data_ptr(), snake[1].data_ptr(), snake[2].data_ptr()
         args.w, args.bias = rec.packed.data_ptr(), _ptr(rec.bias)
         args.res, args.out = _ptr(res), out.data_ptr()
         args.out_batch, args.out_chunk, args.out_row = out_strides
@@ -493,17 +472,17 @@ class Engine:
         args.out_is_16, args.res_is_16, args.fp16 = int(out_bf16), int(res_bf16), self.fp16
         args.alpha, args.beta_res, args.accumulate, args.geglu = alpha, beta, int(accumulate), int(geglu)
         args.act = int(act)
-        args.two_cta = 1 if (rec.two_cta and xf is None) else 0
+        args.two_cta = 1 if rec.two_cta else 0
         args.acc_src = _ptr(acc_src)
         args.B, args.L, args.Cin, args.Cout = B, L, rec.cin_pad, rec.cout_pad
         args.ntaps, args.P, args.tap_off, args.bn = rec.ntaps, rec.P, rec.off_c, rec.bn
         flops = 2.0 * B * L * rec.P * rec.ntaps * rec.cin * rec.cout
         esz_o = 2 if out_bf16 else 4
-        nbytes = B * L * rec.cin * (4 if (xf is not None and not x16) else 2) + B * L * rec.P * rec.cout * (esz_o + ((4 if acc_src is not None else esz_o) if accumulate else 0))
+        nbytes = B * L * rec.cin * 2 + B * L * rec.P * rec.cout * (esz_o + ((4 if acc_src is not None else esz_o) if accumulate else 0))
         if res is not None:
             nbytes += B * L * rec.P * rec.cout * (2 if res_bf16 else 4)
         work = {"flops": flops, "bytes": float(nbytes),
-                "tag": f"tc_conv{'+snake' if xf is not None else ''}[Cin{rec.cin},Cout{rec.cout},k{rec.ntaps}x{rec.P}"
+                "tag": f"tc_conv[Cin{rec.cin},Cout{rec.cout},k{rec.ntaps}x{rec.P}"
                        f"{',res' if res is not None else ''}]"}
         self._launch_conv(args, work)
 
@@ -850,35 +829,11 @@ class Engine:
         if not self.tc:
             return self._vocoder_f32(mel)
         B, N, _ = mel.shape
-        ns = min(self.voc_streams, B)
         wave = torch.empty((B, N * self.vcfg.total_upsample), dtype=torch.float32, device=self.device)
         if self.split:
             self._vocoder_tc_split(mel, wave)
-            return wave
-        if ns <= 1:
-            self._vocoder_tc(mel, wave, "")
-            return wave
-        # Clips are independent: run halves of the batch on separate streams, staggered by one kernel,
-        # so that the FP32-pipe-bound snake kernel of one half overlaps the tensor/HBM-bound conv of the other.
-        main = torch.cuda.current_stream(self.device)
-        ev0 = torch.cuda.Event()
-        ev0.record(main)
-        while len(self._side_streams) < ns:
-            self._side_streams.append(torch.cuda.Stream(self.device))
-        bounds = [B * i // ns for i in range(ns + 1)]
-        prev_started = None
-        for i in range(ns):
-            st = self._side_streams[i]
-            st.wait_event(ev0)
-            if prev_started is not None:
-                st.wait_event(prev_started)
-            started = torch.cuda.Event()
-            with torch.cuda.stream(st):
-                self._vocoder_tc(mel[bounds[i]: bounds[i + 1]], wave[bounds[i]: bounds[i + 1]], f"s{i}", started)
-            prev_started = started
-            done = torch.cuda.Event()
-            done.record(st)
-            main.wait_event(done)
+        else:
+            self._vocoder_tc(mel, wave)
         return wave
 
     def _conv_f32(self, rec: _F32Weight, x, out, B, L, res=None, beta=0.0, alpha=1.0, accumulate=0):
@@ -948,16 +903,14 @@ class Engine:
         t = self.buf(f"{name}@{L}", (B * bs + 4096,), dtype)
         return t, cs, bs
 
-    def _vocoder_tc(self, mel: torch.Tensor, wave: torch.Tensor, tag: str, started_event=None):
+    def _vocoder_tc(self, mel: torch.Tensor, wave: torch.Tensor):
         v, V, st = self.vcfg, self.voc, self.stream
         B, N, nm = mel.shape
         bf, f32 = self.h16, torch.float32
-        _cb = self._cbuf
-        self_cbuf = lambda name, *a: _cb(name + tag, *a)
-        melc, mcs, mbs = self_cbuf("vt_mel", B, nm, N, bf)
+        melc, mcs, mbs = self._cbuf("vt_mel", B, nm, N, bf)
         self._call("fh_to_chunked_16", mel.data_ptr(), N * nm, 1, nm, melc.data_ptr(), mbs, mcs, HALO, B, nm, N, self.fp16, st)
         C0 = self.cpad(v.upsample_initial_channel)
-        xb, xcs, xbs = self_cbuf("vt_pre", B, C0, N, bf)
+        xb, xcs, xbs = self._cbuf("vt_pre", B, C0, N, bf)
         self._tc_conv(V["conv_pre"], melc, mbs, mcs, HALO, xb[HALO * 8:], (xbs, xcs, 8), 1, B, N)
         L = N
         nk = v.num_kernels
@@ -967,7 +920,7 @@ class Engine:
         # 2 ms per step cheaper than separate outputs + a sum pass).  Small batches do not fill 148 SMs: there each
         # branch writes its own pre-scaled output on its own stream (parallel CUDA-graph branches when captured) and
         # fh_sum_cast_f32 adds them.
-        par = (self.branch_streams and B <= self.branch_streams_max_batch and started_event is None and nk > 1)
+        par = (self.branch_streams and B <= self.branch_streams_max_batch and nk > 1)
         main = torch.cuda.current_stream(self.device)
         if par:
             while len(self._branch_streams) < nk:
@@ -975,30 +928,28 @@ class Engine:
         for s, u in enumerate(v.upsample_rates):
             ch = self.cpad(v.stage_channels(s))
             Lo = L * u
-            X, cs, bs = self_cbuf(f"vt_X{s}", B, ch, Lo, f32)
+            X, cs, bs = self._cbuf(f"vt_X{s}", B, ch, Lo, f32)
             o = HALO * 8  # element offset of row t = 0
             strides = (bs, cs, 8)
             self._tc_conv(V[f"up{s}"], a_in, a_bs, a_cs, HALO, X[o:], strides, 0, B, L)
             L = Lo
-            # HBM-bound stages (<= 128 channels, one N tile): the snake runs inside the conv kernel as its A-producer
-            fuse = self.fuse_snake and ch <= 128 and all(V[f"r{s}.{j}.c1.0"].bn >= ch for j in range(nk))
             if par:
                 ev_up = torch.cuda.Event()
                 ev_up.record(main)
             outs = []
             # sequential branches: the last one adds the running mean (XS, fp32) and writes the stage output directly as
             # the 16-bit operand of the next upsampler -- no fp32 store of the mean, no separate cast pass
-            fuse_cast = (not par and nk > 1 and s + 1 < v.num_stages and _os_environ_get("FH_FUSE_CAST", "1") != "0")
+            fuse_cast = not par and nk > 1 and s + 1 < v.num_stages
             if fuse_cast:
-                XBf, _, _ = self_cbuf(f"vt_XB{s}", B, ch, Lo, bf)
+                XBf, _, _ = self._cbuf(f"vt_XB{s}", B, ch, Lo, bf)
             for j, dil in enumerate(v.resblock_dilation_sizes):
                 bt = f"_{j}" if par else ""  # parallel branches need their own scratch
-                XJ, _, _ = self_cbuf(f"vt_XJ{s}{bt}", B, ch, Lo, f32)
-                y16 = (self.y16 or fuse) and v.resblock == "1"  # the tensor between the two convs of a unit is fp16
-                Y, _, _ = self_cbuf(f"vt_Y{s}{bt}" + ("h" if y16 else ""), B, ch, Lo, bf if y16 else f32)
-                A = None if fuse else self_cbuf(f"vt_A{s}{bt}", B, ch, Lo, bf)[0]
+                XJ, _, _ = self._cbuf(f"vt_XJ{s}{bt}", B, ch, Lo, f32)
+                y16 = self.y16 and v.resblock == "1"  # the tensor between the two convs of a unit is fp16
+                Y, _, _ = self._cbuf(f"vt_Y{s}{bt}" + ("h" if y16 else ""), B, ch, Lo, bf if y16 else f32)
+                A = self._cbuf(f"vt_A{s}{bt}", B, ch, Lo, bf)[0]
                 # parallel branches write their own output (summed below); sequential ones accumulate in place
-                XSj, _, _ = self_cbuf(f"vt_XS{s}_{j}" if par else f"vt_XS{s}", B, ch, Lo, f32)
+                XSj, _, _ = self._cbuf(f"vt_XS{s}_{j}" if par else f"vt_XS{s}", B, ch, Lo, f32)
                 outs.append(XSj)
                 ctx = torch.cuda.stream(self._branch_streams[j]) if par else contextlib.nullcontext()
                 if par:
@@ -1009,52 +960,42 @@ class Engine:
                     for i in range(len(dil)):
                         last = i == len(dil) - 1
                         sn1 = V[f"r{s}.{j}.a1.{i}"]
-                        if not fuse:
-                            self._call("fh_snake_aa_chunked", cur.data_ptr(), A.data_ptr(), sn1[0].data_ptr(), sn1[1].data_ptr(),
-                                       sn1[2].data_ptr(), bs, cs, HALO, B, ch, L, self.k16, st)
-                        if started_event is not None:
-                            started_event.record(torch.cuda.current_stream(self.device))
-                            started_event = None
-                        fa = dict(xf=cur, snake=sn1) if fuse else {}
+                        self._call("fh_snake_aa_chunked", cur.data_ptr(), A.data_ptr(), sn1[0].data_ptr(), sn1[1].data_ptr(),
+                                   sn1[2].data_ptr(), bs, cs, HALO, B, ch, L, self.k16, st)
                         if v.resblock == "1":
-                            self._tc_conv(V[f"r{s}.{j}.c1.{i}"], None if fuse else A, bs, cs, HALO, Y[o:], strides,
-                                          1 if y16 else 0, B, L, **fa)
+                            self._tc_conv(V[f"r{s}.{j}.c1.{i}"], A, bs, cs, HALO, Y[o:], strides, 1 if y16 else 0, B, L)
                             sn2 = V[f"r{s}.{j}.a2.{i}"]
-                            if fuse:
-                                pass  # the second snake is the prologue of the second conv (fp16 rows in)
-                            elif y16:
+                            if y16:
                                 self._call("fh_snake_aa_chunked_h", Y.data_ptr(), A.data_ptr(), sn2[0].data_ptr(),
                                            sn2[1].data_ptr(), sn2[2].data_ptr(), bs, cs, HALO, B, ch, L, st)
                             else:
                                 self._call("fh_snake_aa_chunked", Y.data_ptr(), A.data_ptr(), sn2[0].data_ptr(),
                                            sn2[1].data_ptr(), sn2[2].data_ptr(), bs, cs, HALO, B, ch, L, self.k16, st)
-                            fa = dict(xf=Y, snake=sn2, x16=True) if fuse else {}
                             conv = V[f"r{s}.{j}.c2.{i}"]
                         else:
                             conv = V[f"r{s}.{j}.c1.{i}"]
-                        src = None if fuse else A
                         if last and fuse_cast and j == nk - 1:
-                            self._tc_conv(conv, src, bs, cs, HALO, XBf[o:], strides, 1, B, L, res=cur[o:], res_strides=strides,
-                                          alpha=1.0 / nk, beta=1.0 / nk, accumulate=True, acc_src=XSj[o:], **fa)
+                            self._tc_conv(conv, A, bs, cs, HALO, XBf[o:], strides, 1, B, L, res=cur[o:], res_strides=strides,
+                                          alpha=1.0 / nk, beta=1.0 / nk, accumulate=True, acc_src=XSj[o:])
                         elif last:
-                            self._tc_conv(conv, src, bs, cs, HALO, XSj[o:], strides, 0, B, L, res=cur[o:], res_strides=strides,
-                                          alpha=1.0 / nk, beta=1.0 / nk, accumulate=(j > 0 and not par), **fa)
+                            self._tc_conv(conv, A, bs, cs, HALO, XSj[o:], strides, 0, B, L, res=cur[o:], res_strides=strides,
+                                          alpha=1.0 / nk, beta=1.0 / nk, accumulate=(j > 0 and not par))
                         else:
-                            self._tc_conv(conv, src, bs, cs, HALO, XJ[o:], strides, 0, B, L, res=cur[o:], res_strides=strides,
-                                          beta=1.0, **fa)
+                            self._tc_conv(conv, A, bs, cs, HALO, XJ[o:], strides, 0, B, L, res=cur[o:], res_strides=strides,
+                                          beta=1.0)
                             cur = XJ
                     if par:
                         done = torch.cuda.Event()
                         done.record(self._branch_streams[j])
                         main.wait_event(done)
             st = self.stream
-            XS, _, _ = self_cbuf(f"vt_XS{s}", B, ch, Lo, f32)
+            XS, _, _ = self._cbuf(f"vt_XS{s}", B, ch, Lo, f32)
             if par:
                 if len(outs) > 4:
                     raise ValueError("at most 4 resblock kernel sizes per stage")
                 ptrs = [t_.data_ptr() for t_ in outs] + [None] * (4 - len(outs))
             if s + 1 < v.num_stages:
-                XB, _, _ = self_cbuf(f"vt_XB{s}", B, ch, L, bf)
+                XB, _, _ = self._cbuf(f"vt_XB{s}", B, ch, L, bf)
                 if par:
                     self._call("fh_sum_cast_f32", *ptrs, None, XB.data_ptr(), B * bs, self.fp16, st)
                 elif not fuse_cast:
@@ -1062,19 +1003,19 @@ class Engine:
                 a_in, a_cs, a_bs = XB, cs, bs
             elif par:
                 self._call("fh_sum_cast_f32", *ptrs, XS.data_ptr(), None, B * bs, self.fp16, st)
-        self._post(XS, bs, cs, B, ch, L, wave, self_cbuf)
+        self._post(XS, bs, cs, B, ch, L, wave)
 
-    def _post(self, XS, bs, cs, B, ch, L, wave, cbuf):
+    def _post(self, XS, bs, cs, B, ch, L, wave):
         """activation_post -> conv_post -> tanh (bigvgan/models.py:189-192) on the last stage's fp32 rows: one fused kernel
-        (the activated tensor stays in shared memory); FH_FUSE_POST=0 or > 64 channels: two kernels through HBM."""
+        (the activated tensor stays in shared memory); > 64 channels: two kernels through HBM."""
         V, st = self.voc, self.stream
         a, ib, f = V["post_act"]
-        if ch <= 64 and _os_environ_get("FH_FUSE_POST", "1") != "0":
+        if ch <= 64:
             self._call("fh_snakepost_convpost_tanh", XS.data_ptr(), bs, cs, HALO, a.data_ptr(), ib.data_ptr(), f.data_ptr(),
                        V["post_w"].data_ptr(), V["post_b"], wave.data_ptr(), B, ch, L, st,
                        work={"bytes": 4.0 * B * L * (ch + 1), "flops": 2.0 * B * L * ch * (7 + 24)})
             return
-        AP, _, _ = cbuf("vt_AP", B, ch, L, torch.float32)
+        AP, _, _ = self._cbuf("vt_AP", B, ch, L, torch.float32)
         self._call("fh_snake_aa_chunked", XS.data_ptr(), AP.data_ptr(), a.data_ptr(), ib.data_ptr(), f.data_ptr(), bs, cs,
                    HALO, B, ch, L, 0, st)
         self._call("fh_convpost_tanh_chunked", AP.data_ptr(), bs, cs, HALO, V["post_w"].data_ptr(), V["post_b"],
@@ -1134,7 +1075,7 @@ class Engine:
             if s + 1 < v.num_stages:
                 a_in, a_cs, a_bs2 = self._cbuf(f"vs_XB{s}", B, 2 * ch, L, h16)
                 self._call("fh_cast_f32_16_split", XS.data_ptr(), a_in.data_ptr(), cs, ch // 8, bs, a_bs2, B, self.fp16, st)
-        self._post(XS, bs, cs, B, ch, L, wave, self._cbuf)
+        self._post(XS, bs, cs, B, ch, L, wave)
 
     # ------------------------------------------------------------------ stage: post-processing
     def postprocess(self, pred: torch.Tensor, src: torch.Tensor) -> torch.Tensor:
@@ -1150,27 +1091,16 @@ class Engine:
         en = self.buf("pp_en", (B, 1025), zero=False)
         cut = self.buf("pp_cut", (B,), torch.int32)
         frames = self.buf("pp_fr", (B, nt, 2048), zero=False)
-        if self.pp_fused:
-            # no spectrogram in HBM: energy pass over src (two frames per complex FFT), then per frame
-            # FFT(pred + i src) -> split -> splice -> inverse FFT
-            ws = self.buf("pp_ws", (self.lib.fh_pp_energy_ws_bytes(B, NT) // 8,), torch.float64, zero=False)
-            self._call("fh_pp_src_energy_f32", src.data_ptr(), en.data_ptr(), ws.data_ptr(), self.window.data_ptr(),
-                       self.twiddle.data_ptr(), B, T, NT, st, work={"bytes": 4.0 * B * T, "flops": B * NT * 0.5 * 5.0 * 2048 * 11})
-            self._call("fh_pp_cutoff", en.data_ptr(), cut.data_ptr(), B, 0.99, st)
-            # bytes: pred + src read once (algorithmic), windowed frames written (2048 per 480 new samples: the OLA input)
-            self._call("fh_pp_fused_f32", pred.data_ptr(), src.data_ptr(), cut.data_ptr(), frames.data_ptr(),
-                       self.window.data_ptr(), self.twiddle.data_ptr(), B, Tp, T, NT, st,
-                       work={"bytes": 4.0 * B * (Tp + T) + 4.0 * B * NT * 2048, "flops": B * NT * 2.0 * 5.0 * 2048 * 11})
-        else:
-            sp = self.buf("pp_sp", (B, NTp, 1025, 2), zero=False)
-            ss = self.buf("pp_ss", (B, NT, 1025, 2), zero=False)
-            self._call("fh_stft_center_f32", pred.data_ptr(), sp.data_ptr(), None, self.window.data_ptr(),
-                       self.twiddle.data_ptr(), B, Tp, NTp, st)
-            self._call("fh_stft_center_f32", src.data_ptr(), ss.data_ptr(), en.data_ptr(), self.window.data_ptr(),
-                       self.twiddle.data_ptr(), B, T, NT, st)
-            self._call("fh_pp_cutoff", en.data_ptr(), cut.data_ptr(), B, 0.99, st)
-            self._call("fh_pp_splice_istft_f32", sp.data_ptr(), ss.data_ptr(), cut.data_ptr(), frames.data_ptr(),
-                       self.window.data_ptr(), self.twiddle.data_ptr(), B, nt, st)
+        # no spectrogram in HBM: energy pass over src (two frames per complex FFT), then per frame
+        # FFT(pred + i src) -> split -> splice -> inverse FFT
+        ws = self.buf("pp_ws", (self.lib.fh_pp_energy_ws_bytes(B, NT) // 8,), torch.float64, zero=False)
+        self._call("fh_pp_src_energy_f32", src.data_ptr(), en.data_ptr(), ws.data_ptr(), self.window.data_ptr(),
+                   self.twiddle.data_ptr(), B, T, NT, st, work={"bytes": 4.0 * B * T, "flops": B * NT * 0.5 * 5.0 * 2048 * 11})
+        self._call("fh_pp_cutoff", en.data_ptr(), cut.data_ptr(), B, 0.99, st)
+        # bytes: pred + src read once (algorithmic), windowed frames written (2048 per 480 new samples: the OLA input)
+        self._call("fh_pp_fused_f32", pred.data_ptr(), src.data_ptr(), cut.data_ptr(), frames.data_ptr(),
+                   self.window.data_ptr(), self.twiddle.data_ptr(), B, Tp, T, NT, st,
+                   work={"bytes": 4.0 * B * (Tp + T) + 4.0 * B * NT * 2048, "flops": B * NT * 2.0 * 5.0 * 2048 * 11})
         y = self.buf("pp_y", (B, T), zero=False)
         absmax = self.buf("pp_absmax", (B,), torch.int32)
         self._call("fh_fill_u32", absmax.data_ptr(), 0, B, st)

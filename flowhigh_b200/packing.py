@@ -87,13 +87,6 @@ def f32_conv_buffers(tc: TappedConv, device):
 
 
 def pick_bn(cout_pad: int) -> int:
-    import os
-    ov = os.environ.get("FH_BN_OVERRIDE")  # e.g. "192:96,384:128" (tuning experiments)
-    if ov:
-        for item in ov.split(","):
-            k, v = item.split(":")
-            if int(k) == cout_pad:
-                return int(v)
     # Measured on B200 once the MMA issue loop stopped pacing the kernel (gpurun_out/bd5_*.json): accumulators that fit
     # TMEM twice (2 sub-tiles x bn <= 256 columns) so the epilogue overlaps the next tile beat the wider single-buffered
     # tiles for 192 and 384 output channels (-12 % / -21 %); 768 keeps 3 x 256.

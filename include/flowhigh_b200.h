@@ -76,14 +76,8 @@ int fh_stft_logmel_f32(const float* audio, float* mel, const float* window, cons
 
 /* ---------------------------------------------------------------- post-processing
  * replaces PostProcessing.post_processing   postprocessing.py:18-41
- * fh_stft_center: complex STFT (n_fft = win = 2048, hop 480, periodic Hann, center, ZERO pad):
- *   x [B,T] -> spec [B, NT, 1025] float2, NT = 1 + T/480; energy (may be NULL) [B,1025] gets
- *   sum_t |S[f,t]| accumulated with atomics (caller zeroes it). */
-int fh_stft_center_f32(const float* x, float* spec, float* energy, const float* window,
-                       const float* twiddle, int B, int T, int NT, void* stream);
-/* cutoff[b] = postprocessing.py:10-16 applied to energy[b,:] (cumsum, 0.99 threshold) */
-int fh_pp_cutoff(const float* energy, int* cutoff, int B, float threshold, void* stream);
-/* Fused form of the same post-processing (no spectrogram in HBM; two real frames per complex FFT):
+ * STFT: n_fft = win = 2048, hop 480, periodic Hann, center, ZERO pad; NT = 1 + T/480 frames.
+ * No spectrogram reaches HBM: two real frames share one complex FFT.
  * fh_pp_src_energy: energy[B,1025] = sum_t |STFT(src)| (workspace of fh_pp_energy_ws_bytes(B, NT) bytes, 8-byte aligned);
  * fh_pp_fused: per frame STFT(pred), STFT(src) -> splice at cutoff[b] -> inverse FFT -> windowed frames [B,NT,2048]
  * for fh_pp_overlap_add_f32.  pred [B,Tp] and src [B,T] must span the same NT = 1 + T/480 frames. */
@@ -92,10 +86,8 @@ int fh_pp_src_energy_f32(const float* src, float* energy, void* workspace, const
                          int B, int T, int NT, void* stream);
 int fh_pp_fused_f32(const float* pred, const float* src, const int* cutoff, float* frames, const float* window,
                     const float* twiddle, int B, int Tp, int T, int NT, void* stream);
-/* frames [B,NT,2048] = window * irfft(f < cutoff[b] ? spec_src : spec_pred) */
-int fh_pp_splice_istft_f32(const float* spec_pred, const float* spec_src, const int* cutoff,
-                           float* frames, const float* window, const float* twiddle,
-                           int B, int NT, void* stream);
+/* cutoff[b] = postprocessing.py:10-16 applied to energy[b,:] (cumsum, 0.99 threshold) */
+int fh_pp_cutoff(const float* energy, int* cutoff, int B, float threshold, void* stream);
 /* y[b,t] = OLA(frames)[t+1024] / OLA(window^2)[t+1024] for t < length (torch.istft semantics) */
 int fh_pp_overlap_add_f32(const float* frames, float* y, const float* window, uint32_t* absmax_bits,
                           int B, int NT, int length, void* stream);
@@ -245,20 +237,10 @@ typedef struct {
   const int* tap_off;     /* HOST pointer [P][ntaps] row offsets */
   int bn;                 /* N tile, multiple of 16, <= 256 */
   int fp16;               /* 16-bit operand format: 0 = bfloat16, 1 = IEEE half (same rate, 3 more mantissa bits) */
-  /* fused anti-aliased Snake prologue (optional): when x_f32 != NULL the A operand is Activation1d(x) computed inside
-   * the kernel (alias_free_torch/act.py:23-28 + bigvgan/models.py:63-72 `conv(act(x))`) and never written to HBM;
-   * x is chunked fp32 -- or fp16 rows when x_is_16 != 0 -- with the geometry a_batch / a_chunk / a_row0 describe
-   * (>= 8 zero rows are NOT required: windows are clipped to the buffer and replicate-patched); `a` is ignored.
-   * Needs fp16 operands, P == 1, Cin <= 128 and Cout <= bn <= 128. */
-  const void* x_f32;
-  const float* sn_a;      /* [Cin] alpha (already exp'd when logscale) */
-  const float* sn_inv_b;  /* [Cin] 1 / (beta + 1e-9) */
-  const float* sn_filt;   /* [12] Kaiser-sinc taps */
   int act;                /* 0 none, 1 exact-erf GELU on (acc + bias) * alpha, before the residual (convnext.py:56-57) */
   const float* acc_src;   /* accumulate != 0: rows to add, fp32 with the output geometry; NULL = the output itself.
                            * Lets the last AMP branch of a stage (bigvgan/models.py:181-187, xs / num_kernels) write the
                            * mean directly as the 16-bit operand of the next upsampler (out_is_16 = 1). */
-  int x_is_16;            /* fused prologue: x_f32 points to fp16 rows (the 16-bit output of the unit's first conv) */
   int two_cta;            /* CTA-pair kernel (tcgen05 cta_group::2, M = 256): `w` must be packed per CTA rank
                            * ([p][nt][ci-pair][rank][tap][2][bn/2][8], packing.pack_tc(two_cta=True)) */
 } fh_tc_conv_args;

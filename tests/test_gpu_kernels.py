@@ -73,26 +73,20 @@ def test_logmel(cuda_device, sr, precise):
         assert l1_64 <= 2 * floor + 1e-5
 
 
-@pytest.mark.parametrize("fused", [True, False])
-def test_postprocess(cuda_device, fused):
-    """fused: spectrogram-free path (two real frames per complex FFT, splice + inverse FFT per frame);
-    unfused: STFT(pred), STFT(src) to HBM, energy, splice + iSTFT -- both against the oracle."""
+def test_postprocess(cuda_device):
+    """Spectrogram-free post-processing (two real frames per complex FFT, splice + inverse FFT per frame) against the
+    oracle."""
     eng, *_ = engine("gen_basic_midpoint", "fp32")
     torch.manual_seed(0)
-    prev = eng.pp_fused
-    eng.pp_fused = fused
-    try:
-        for T in (480 * 30, 480 * 30 + 123, 480 * 37 + 1):  # odd and even frame counts, pred shorter than src
-            Tp = T // 480 * 480
-            src = torch.from_numpy(np.stack([synth_speech(T, 48000, 3), synth_speech(T, 48000, 4) * 0.5]))
-            pred = torch.randn(2, Tp) * 0.1
-            out = eng.postprocess(pred.cuda(), src.cuda()).cpu()
-            for i in range(2):
-                ref = dsp.postprocess(pred[i:i + 1], src[i:i + 1], T)
-                assert float((out[i:i + 1] - ref).abs().max()) <= 2e-5
-                assert abs(float(out[i].abs().max()) - 0.99) < 1e-6
-    finally:
-        eng.pp_fused = prev
+    for T in (480 * 30, 480 * 30 + 123, 480 * 37 + 1):  # odd and even frame counts, pred shorter than src
+        Tp = T // 480 * 480
+        src = torch.from_numpy(np.stack([synth_speech(T, 48000, 3), synth_speech(T, 48000, 4) * 0.5]))
+        pred = torch.randn(2, Tp) * 0.1
+        out = eng.postprocess(pred.cuda(), src.cuda()).cpu()
+        for i in range(2):
+            ref = dsp.postprocess(pred[i:i + 1], src[i:i + 1], T)
+            assert float((out[i:i + 1] - ref).abs().max()) <= 2e-5
+            assert abs(float(out[i].abs().max()) - 0.99) < 1e-6
 
 
 # ------------------------------------------------------------------ fp32 kernels
@@ -118,7 +112,7 @@ def test_snake_chunked(cuda_device, out_kind):
     """fh_snake_aa_chunked on the chunked [C/8][Lp][8] layout against the oracle closed form: fp16 output (Toeplitz-MMA
     kernel; out_kind 3 = fh_snake_aa_chunked_h, the same kernel fed with fp16 rows through ldmatrix), bf16 and fp32
     output (scalar kernel).  Lengths cover one-tile, multi-tile, tile-boundary (512 / 544 rows)
-    and shorter-than-the-filter sequences (tile = 1024 rows by default, 512 with FH_SNAKE_NB=8, 544 for the scalar kernel); the rows after L must stay untouched (they are the next conv's zero padding)."""
+    and shorter-than-the-filter sequences (tile = 1024 rows for the MMA kernel, 544 for the scalar kernel); the rows after L must stay untouched (they are the next conv's zero padding)."""
     eng, sd, vcfg, _ = engine("gen_basic_midpoint", "fp32")
     torch.manual_seed(5)
     filt = torch.from_numpy(np.ascontiguousarray(eng.sd["flowhigh.audio_enc_dec.vocoder.activation_post.upsample.filter"].cpu().numpy()))
@@ -643,30 +637,6 @@ def test_generate_rejects_too_short_clip(cuda_device, f32_model):
     m, _ = f32_model
     with pytest.raises(ValueError):
         m.generate(np.zeros(100, np.float32) + 0.1, 16000, 48000)  # 300 samples @ 48 k < 785
-
-
-@pytest.mark.parametrize("name", ["voc_resblock2_snake", "voc_resblock1_snakebeta"])
-def test_fused_snake_conv_matches_unfused(cuda_device, name):
-    """tc_conv_snakepro_kernel (the Toeplitz-MMA snake as the in-kernel producer of the conv's A operand, fp32 and fp16
-    row inputs, aligned windows with m_valid = 128 msub - span rows per tile) against the separate snake launches."""
-    eng, sd, vcfg, g = engine(name, "fp16")
-    mel = dev(g["mel"])
-    prev = eng.fuse_snake
-    try:
-        eng.fuse_snake = False
-        a = eng.vocoder(mel).cpu()
-        eng.fuse_snake = True
-        b = eng.vocoder(mel).cpu()
-    finally:
-        eng.fuse_snake = prev
-    # The two paths round differently (snake FMA order, bias folded into an FMA in the specialised epilogue); a
-    # rounding-level change upstream flips 16-bit operand roundings downstream, so they agree only to the 16-bit
-    # operand error itself (max-abs ~2e-3 vs fp64 for either path).  Both must sit at the same distance from fp64.
-    ref = torch.from_numpy(g["f64_vocoder"]).reshape(a.shape).float()
-    err = float((a - b).abs().max())
-    sa, sb = snr_db(ref, a), snr_db(ref, b)
-    print(f"fused snake+conv vs unfused {name}: max-abs {err:.3g}, SNR vs fp64 {sa:.2f} / {sb:.2f} dB")
-    assert err <= 3e-3 and sa >= 55.0 and sb >= 55.0 and abs(sa - sb) <= 2.0
 
 
 @pytest.mark.parametrize("name", ["voc_resblock1_snakebeta", "voc_resblock2_snake"])

@@ -60,16 +60,14 @@ SIGNATURES = {
     "fh_dwconv_gelu_res_f32": (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _p]),
     "fh_dwconv_f32": (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _p]),
     "fh_layernorm_f32": (_i, [_p, _p, _p, _p, _i, _i64, _i, _i, _f, _p]),
-    "fh_gelu_f32": (_i, [_p, _p, _i, _i64, _i, _i, _p]),
+    "fh_gelu_f32": (_i, [_p, _p, _i, _i, _p]),
     "fh_rmsnorm_f32": (_i, [_p, _p, _p, _p, _i, _i64, _i, _i, _p]),
     "fh_qknorm_rope_f32": (_i, [_p, _p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _p]),
-    "fh_attention_f32": (_i, [_p, _p, _p, _p, _i, _i64, _i, _i, _i, _i, _f, _p]),
-    "fh_qknorm_rope_split": (_i, [_p, _p, _p, _p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _f, _i, _p]),
-    "fh_attention_tc": (_i, [_p, _p, _p, _p, _p, _p, _i, _i64, _i, _i, _i, _i, _i, _p]),
+    "fh_attention_f32": (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _f, _p]),
     "fh_attention_tc5_operand_elems": (_i64, [_i, _i, _i, _i]),
     "fh_qknorm_rope_tiles": (_i, [_p, _p, _p, _p, _p, _p, _p, _i, _i, _i, _i, _f, _i, _p]),
     "fh_attention_tc5": (_i, [_p, _p, _p, _p, _i, _i64, _i, _i, _i, _i, _i, _p]),
-    "fh_geglu_f32": (_i, [_p, _p, _i, _i64, _i, _i, _i, _p]),
+    "fh_geglu_f32": (_i, [_p, _p, _i, _i, _p]),
     "fh_axpby_f32": (_i, [_p, _p, _f, _f, _p, _i64, _p]),
     "fh_rk_lincomb_f32": (_i, [_p, _p, _i64, _i, C.POINTER(_f), _p, _i64, _p]),
     "fh_rk_scaled_sumsq_f32": (_i, [_p, _p, _p, _f, _f, _i, _i64, _p, _p]),

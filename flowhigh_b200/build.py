@@ -16,7 +16,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIBNAME = "libflowhigh_b200.so"
-SOURCES = ["dsp.cu", "backbone.cu", "vocoder_f32.cu", "vocoder_tc.cu", "tc_conv.cu", "attention_tc.cu", "attention_tc5.cu"]
+SOURCES = ["dsp.cu", "backbone.cu", "vocoder_f32.cu", "vocoder_tc.cu", "tc_conv.cu", "attention_tc5.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden"]
 

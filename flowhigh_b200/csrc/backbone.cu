@@ -178,15 +178,11 @@ __global__ void layernorm_kernel(const float* __restrict__ x, const float* __res
   }
 }
 
-// exact-erf GELU, fp32 row-major in -> fp32 row-major (out_mode 0) or 16-bit chunked (nn.GELU, convnext.py:36)
-__global__ void gelu_kernel(const float* __restrict__ x, void* __restrict__ out, int out_mode, int64_t out_rows, int M, int C,
-                            unsigned int* status) {
+// exact-erf GELU, fp32 row-major (nn.GELU, convnext.py:36)
+__global__ void gelu_kernel(const float* __restrict__ x, float* __restrict__ out, int M, int C) {
   const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= (long long)M * C) return;
-  const int row = (int)(i / C), c = (int)(i % C);
-  const float y = fh::gelu_erf(x[i]);
-  if (out_mode == 0) ((float*)out)[i] = y;
-  else ((unsigned short*)out)[fh::chunked_index(out_rows * 8, row, c)] = fh::cvt16_guard(y, out_mode == 2, status);
+  out[i] = fh::gelu_erf(x[i]);
 }
 
 // ------------------------------------------------------------------------------ (adaptive) RMS norm
@@ -259,9 +255,8 @@ __global__ void qknorm_rope_kernel(const float* __restrict__ qkv, const float* _
 // softmax(scale q k^T) v, no mask.  One CTA per (64 queries, b*h); keys streamed in blocks of 64;
 // online softmax.  256 threads: thread (ty, tx) owns S/O rows 4*ty..+3, cols 4*tx..+3.
 __global__ void __launch_bounds__(256) attention_f32_kernel(const float* __restrict__ Q, const float* __restrict__ Kt,
-                                                            const float* __restrict__ V, void* __restrict__ out,
-                                                            int out_mode, int64_t out_rows, int H, int N, float scale,
-                                                            unsigned int* status) {
+                                                            const float* __restrict__ V, float* __restrict__ out, int H,
+                                                            int N, float scale) {
   constexpr int D = 64, BQ = 64, BK = 64;
   extern __shared__ __align__(16) float att_smem[];
   float (*Qs)[BQ + 1] = reinterpret_cast<float (*)[BQ + 1]>(att_smem);                      // [d][q]
@@ -352,33 +347,17 @@ __global__ void __launch_bounds__(256) attention_f32_kernel(const float* __restr
     const float inv = 1.0f / lrow[i];
     const int64_t row = (int64_t)bi * N + qi;
 #pragma unroll
-    for (int j = 0; j < 4; ++j) {
-      const int c = h * D + tx * 4 + j;
-      const float val = o[i][j] * inv;
-      if (out_mode == 0)
-        ((float*)out)[row * (H * D) + c] = val;
-      else
-        ((unsigned short*)out)[fh::chunked_index(out_rows * 8, row, c)] = fh::cvt16_guard(val, out_mode == 2, status);
-    }
+    for (int j = 0; j < 4; ++j) out[row * (H * D) + h * D + tx * 4 + j] = o[i][j] * inv;
   }
 }
 
 // ------------------------------------------------------------------------------ GEGLU / axpby
-__global__ void geglu_kernel(const float* __restrict__ u, void* __restrict__ g, int out_mode, int64_t out_rows, int M,
-                             int inner, int inner_pad, unsigned int* status) {
+__global__ void geglu_kernel(const float* __restrict__ u, float* __restrict__ g, int inner) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   const int m = blockIdx.y;
-  if (i >= inner_pad) return;
-  float v = 0.f;
-  if (i < inner) {
-    const float* ur = u + (size_t)m * 2 * inner;
-    v = fh::gelu_erf(ur[inner + i]) * ur[i];
-  }
-  if (out_mode == 0) {
-    if (i < inner) ((float*)g)[(size_t)m * inner + i] = v;
-  } else {
-    ((unsigned short*)g)[fh::chunked_index(out_rows * 8, m, i)] = fh::cvt16_guard(v, out_mode == 2, status);
-  }
+  if (i >= inner) return;
+  const float* ur = u + (size_t)m * 2 * inner;
+  g[(size_t)m * inner + i] = fh::gelu_erf(ur[inner + i]) * ur[i];
 }
 
 __global__ void axpby_kernel(const float* __restrict__ x, const float* __restrict__ z, float a, float b,
@@ -527,12 +506,10 @@ extern "C" __attribute__((visibility("default"))) int fh_layernorm_f32(const flo
   return fh::check_launch("fh_layernorm_f32");
 }
 
-extern "C" __attribute__((visibility("default"))) int fh_gelu_f32(const float* x, void* out, int out_mode, int64_t out_rows, int M, int C,
-                           void* stream) {
-  FH_REQUIRE(M > 0 && C > 0 && (out_mode == 0 || (C % 8 == 0 && out_rows >= M)), FH_ERR_BAD_SHAPE, "fh_gelu_f32: bad shape");
+extern "C" __attribute__((visibility("default"))) int fh_gelu_f32(const float* x, float* out, int M, int C, void* stream) {
+  FH_REQUIRE(M > 0 && C > 0, FH_ERR_BAD_SHAPE, "fh_gelu_f32: bad shape");
   const long long n = (long long)M * C;
-  gelu_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(x, out, out_mode, out_rows, M, C,
-                                                                               fh::status_word());
+  gelu_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(x, out, M, C);
   return fh::check_launch("fh_gelu_f32");
 }
 
@@ -554,43 +531,29 @@ extern "C" __attribute__((visibility("default"))) int fh_qknorm_rope_f32(const f
   return fh::check_launch("fh_qknorm_rope_f32");
 }
 
-extern "C" __attribute__((visibility("default"))) int fh_attention_f32(const float* q, const float* k, const float* v, void* out, int out_mode,
-                                int64_t out_rows, int B, int H, int N, int D, float scale, void* stream) {
+extern "C" __attribute__((visibility("default"))) int fh_attention_f32(const float* q, const float* k, const float* v, float* out, int B,
+                                int H, int N, int D, float scale, void* stream) {
   FH_REQUIRE(D == 64, FH_ERR_UNSUPPORTED_CFG, "fh_attention_f32: dim_head must be 64 (got %d)", D);
   FH_REQUIRE(B * H <= 65535, FH_ERR_BAD_SHAPE, "fh_attention_f32: B*H must be <= 65535");
   constexpr int kAttSmem = (3 * 64 * 65 + 64 * 68) * (int)sizeof(float);
   static int smem_set[64] = {0};
   fh::ensure_dyn_smem(attention_f32_kernel, kAttSmem, smem_set);
-  attention_f32_kernel<<<dim3((N + 63) / 64, B * H), 256, kAttSmem, (cudaStream_t)stream>>>(q, k, v, out, out_mode, out_rows, H,
-                                                                                   N, scale, fh::status_word());
+  attention_f32_kernel<<<dim3((N + 63) / 64, B * H), 256, kAttSmem, (cudaStream_t)stream>>>(q, k, v, out, H, N, scale);
   return fh::check_launch("fh_attention_f32");
 }
 
-extern "C" __attribute__((visibility("default"))) int fh_geglu_f32(const float* u, void* g, int out_mode, int64_t out_rows, int M, int inner, int inner_pad,
-                            void* stream) {
-  FH_REQUIRE(M > 0 && inner > 0 && inner_pad >= inner && M <= 2147483647, FH_ERR_BAD_SHAPE, "fh_geglu_f32: bad shape");
+extern "C" __attribute__((visibility("default"))) int fh_geglu_f32(const float* u, float* g, int M, int inner, void* stream) {
+  FH_REQUIRE(M > 0 && inner > 0, FH_ERR_BAD_SHAPE, "fh_geglu_f32: bad shape");
   FH_REQUIRE(M <= 65535 * 1024, FH_ERR_BAD_SHAPE, "fh_geglu_f32: M too large");
-  // grid.y limited to 65535: fold rows into blocks of y
-  dim3 grid((inner_pad + 255) / 256, M);
-  if (M > 65535) {
-    // split into several launches
-    int done = 0;
-    while (done < M) {
-      int cnt = M - done > 65535 ? 65535 : M - done;
-      const float* uu = u + (size_t)done * 2 * inner;
-      void* gg = out_mode == 0 ? (void*)((float*)g + (size_t)done * inner)
-                               : (void*)((__nv_bfloat16*)g + (size_t)done * 8);
-      geglu_kernel<<<dim3(grid.x, cnt), 256, 0, (cudaStream_t)stream>>>(uu, gg, out_mode, out_rows, cnt, inner,
-                                                                        inner_pad, fh::status_word());
-      int rc = fh::check_launch("fh_geglu_f32");
-      if (rc) return rc;
-      done += cnt;
-    }
-    return FH_OK;
+  // grid.y is limited to 65535: rows beyond it go to further launches
+  for (int done = 0; done < M; done += 65535) {
+    const int cnt = M - done > 65535 ? 65535 : M - done;
+    geglu_kernel<<<dim3((inner + 255) / 256, cnt), 256, 0, (cudaStream_t)stream>>>(u + (size_t)done * 2 * inner,
+                                                                                  g + (size_t)done * inner, inner);
+    const int rc = fh::check_launch("fh_geglu_f32");
+    if (rc) return rc;
   }
-  geglu_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(u, g, out_mode, out_rows, M, inner, inner_pad,
-                                                       fh::status_word());
-  return fh::check_launch("fh_geglu_f32");
+  return FH_OK;
 }
 
 extern "C" __attribute__((visibility("default"))) int fh_axpby_f32(const float* x, const float* z, float a, float b, float* y, int64_t n, void* stream) {

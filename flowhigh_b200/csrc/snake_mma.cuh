@@ -23,9 +23,6 @@
 #pragma once
 #include <cuda_fp16.h>
 #include "snake_worker.cuh"
-#ifndef FH_SNAKE_K8
-#define FH_SNAKE_K8 1  // edge terms of the down filter as K = 8 MMAs (0: all three terms K = 16; A/B builds only)
-#endif
 
 namespace fh {
 
@@ -252,11 +249,7 @@ __device__ __forceinline__ void snake_mma_unit(const SnakeFrags& F, float* xw, u
       // terms are K = 8 MMAs on half of the A fragment (the other half of the Toeplitz fragment is identically zero).
       if (j >= 1) {  // last term of down block j - 1 (first 8 up-samples of step j), then store it
         float (&yy)[4] = y[(j - 1) % 3];
-#if FH_SNAKE_K8
         sm_mma_k8(yy, U[0], U[1], F.bd[2][0], yy[0], yy[1], yy[2], yy[3]);
-#else
-        sm_mma(yy, U[0], U[1], U[2], U[3], F.bd[2][0], F.bd[2][1], yy[0], yy[1], yy[2], yy[3]);
-#endif
       }
       if (j >= 0 && j < NB) {
         float (&yy)[4] = y[j % 3];
@@ -264,11 +257,7 @@ __device__ __forceinline__ void snake_mma_unit(const SnakeFrags& F, float* xw, u
       }
       if (j + 1 < NB) {  // first term of down block j + 1 (last 8 up-samples of step j)
         float (&yy)[4] = y[(j + 1) % 3];
-#if FH_SNAKE_K8
         sm_mma_k8(yy, U[2], U[3], F.bd[0][1], hib, hib, hib, hib);
-#else
-        sm_mma(yy, U[0], U[1], U[2], U[3], F.bd[0][0], F.bd[0][1], hib, hib, hib, hib);
-#endif
       }
       if (j >= 1) {
         // outputs q0 + 8 i + {2 q, 2 q + 1} of channel g, both halves: the accumulator tile is an 8 x 8 [seq][time]

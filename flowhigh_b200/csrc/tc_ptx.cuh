@@ -32,29 +32,12 @@ __device__ __forceinline__ bool mbar_try(uint32_t bar, uint32_t parity) {
       : "memory");
   return ok != 0;
 }
-// try_wait with a suspend-time hint (ns): the waiting warp sleeps until the phase completes (or the hint expires) instead
-// of spinning -- a spinning warp takes issue slots from the working warps of its scheduler (snake kernel: 10 % of all
-// executed instructions were spin iterations; the hint alone took 10 % off its time)
-#ifndef FH_MBAR_SLEEP_NS
-#define FH_MBAR_SLEEP_NS 0  // measured neutral in the tcgen05 kernels (283.1 - 283.2 vs 283.3 - 285.3 ms per step): plain try_wait stays the default
-#endif
-__device__ __forceinline__ bool mbar_try_sleep(uint32_t bar, uint32_t parity) {
-  if (FH_MBAR_SLEEP_NS == 0) return mbar_try(bar, parity);
-  uint32_t ok;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3;\n\t"
-      "selp.b32 %0, 1, 0, p;\n\t}"
-      : "=r"(ok)
-      : "r"(bar), "r"(parity), "r"((uint32_t)FH_MBAR_SLEEP_NS)
-      : "memory");
-  return ok != 0;
-}
-// bounded wait: a protocol bug becomes a trap (reported as a launch failure), not a hung GPU
+// bounded wait: a protocol bug becomes a trap (reported as a launch failure), not a hung GPU.  The wait spins on plain
+// try_wait: a suspend-time hint measured neutral in the tcgen05 kernels (DESIGN.md §4).
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity, unsigned int* err_flag, int code) {
   if (mbar_try(bar, parity)) return;
   const long long t0 = clock64();
-  while (!mbar_try_sleep(bar, parity)) {
+  while (!mbar_try(bar, parity)) {
     if (clock64() - t0 > 4000000000LL) {
       if (err_flag) {
         atomicExch(err_flag, (unsigned)code | (blockIdx.x << 8) | ((threadIdx.x >> 5) << 24));

@@ -77,9 +77,7 @@ class Engine:
         self._touch_log = None         # {id: object} while a CUDA graph is warmed up / captured: what the graph must keep alive
         self.profile = None
         import os as _os
-        self.tc_attention = _os.environ.get("FH_TC_ATTENTION", "1") != "0"  # tensor-core split-operand attention
         self._cool_ms = float(_os.environ.get("FH_PROFILE_COOL_MS", "0"))
-        self.attn5 = _os.environ.get("FH_ATTN_TC5", "1") != "0"  # tcgen05 / TMEM kernel (0: the mma.sync kernel)
         # fp16 path: the first convolution of an AMP unit writes fp16 rows and the snake behind it reads them as MMA
         # operands (fh_snake_aa_chunked_h) -- the fp32 round trip of that tensor disappears
         self.y16 = self.fp16 and not self.split
@@ -513,9 +511,6 @@ class Engine:
         st = self.stream
         E = self.buf("bb_E", (M, D), zero=False)
         h = self.buf("bb_h", (M, D), zero=False)
-        q = self.buf("bb_q", (B, H, N, Dh), zero=False)
-        k = self.buf("bb_k", (B, H, N, Dh), zero=False)
-        v = self.buf("bb_v", (B, H, N, Dh), zero=False)
         qkv = self.buf("bb_qkv", (M, 3 * D), zero=False)
         if self.tc:
             Mp = packing.round_up(M, 128) + 64
@@ -583,42 +578,31 @@ class Engine:
                 self._call("fh_rmsnorm_f32", h.data_ptr(), tcnd[(l, 2, "gamma")].data_ptr(), tcnd[(l, 2, "beta")].data_ptr(),
                            a.data_ptr(), 0, 0, M, D, st)
                 self._sgemm(a, D, sd[p + "3.to_qkv.weight"], D, None, None, 0, 0.0, 1.0, qkv, 3 * D, M, 3 * D, D)
-            if self.tc and self.tc_attention and self.attn5:
-                # tcgen05 attention: q / k / v^T written directly as the MMA operand images (attention_tc5.cu)
+            if self.tc:
+                # tcgen05 attention: q / k / v^T written directly as the MMA operand images (attention_tc5.cu).  The
+                # profile tags are the names bench.py's attention roofline reads.
                 ops = [self.buf(f"bb_{nm}5", (int(self.lib.fh_attention_tc5_operand_elems(w, B, H, N)),), self.h16)
                        for w, nm in enumerate(("q", "k", "v"))]
                 self._call("fh_qknorm_rope_tiles", qkv.data_ptr(), sd[p + "3.q_norm.gamma"].data_ptr(),
                            sd[p + "3.k_norm.gamma"].data_ptr(), sd[FH + "transformer.rotary_emb.inv_freq"].data_ptr(),
                            *[t_.data_ptr() for t_ in ops], B, N, H, Dh, float(b.qk_norm_scale), self.fp16, st,
                            work={"bytes": (12.0 + 10.0) * B * N * H * Dh, "tag": "fh_qknorm_rope_split"})
+                # algorithmic: q k^T and p v, 2 N^2 Dh each per head; bytes: q (hi + lo), k (hi + lo), v in, out (all 16-bit)
                 self._call("fh_attention_tc5", *[t_.data_ptr() for t_ in ops], act.data_ptr(), self.k16, Mp, B, H, N, Dh,
                            self.fp16, st, work={"flops": 4.0 * B * H * N * N * Dh, "bytes": 2.0 * 6 * B * H * N * Dh,
                                                 "tag": "fh_attention_tc"})
-            elif self.tc and self.tc_attention:
-                s16 = [self.buf(f"bb_{nm}16", (B, H, N, Dh), self.h16, zero=False) for nm in ("qh", "ql", "kh", "kl", "v")]
-                self._call("fh_qknorm_rope_split", qkv.data_ptr(), sd[p + "3.q_norm.gamma"].data_ptr(),
-                           sd[p + "3.k_norm.gamma"].data_ptr(), sd[FH + "transformer.rotary_emb.inv_freq"].data_ptr(),
-                           *[t_.data_ptr() for t_ in s16], B, N, H, Dh, float(b.qk_norm_scale), self.fp16, st,
-                           work={"bytes": (12.0 + 10.0) * B * N * H * Dh})
-                # algorithmic: q k^T and p v, 2 N^2 Dh each per head; bytes: q (hi + lo), k (hi + lo), v in, out (all 16-bit)
-                self._call("fh_attention_tc", *[t_.data_ptr() for t_ in s16], act.data_ptr(), self.k16, Mp, B, H, N, Dh,
-                           self.fp16, st, work={"flops": 4.0 * B * H * N * N * Dh, "bytes": 2.0 * 6 * B * H * N * Dh})
-            else:
-                self._call("fh_qknorm_rope_f32", qkv.data_ptr(), sd[p + "3.q_norm.gamma"].data_ptr(),
-                           sd[p + "3.k_norm.gamma"].data_ptr(), sd[FH + "transformer.rotary_emb.inv_freq"].data_ptr(),
-                           q.data_ptr(), k.data_ptr(), v.data_ptr(), B, N, H, Dh, st)
-                if self.tc:
-                    self._call("fh_attention_f32", q.data_ptr(), k.data_ptr(), v.data_ptr(), act.data_ptr(), self.k16, Mp, B, H,
-                               N, Dh, float(b.qk_norm_scale), st)
-            if self.tc:
                 self._tc_conv(L[f"out{l}"], act, 0, cs, 0, h, rm(D), 0, 1, M, res=h, res_strides=rm(D), beta=1.0)
                 self._call("fh_rmsnorm_f32", h.data_ptr(), tcnd[(l, 4, "gamma")].data_ptr(), tcnd[(l, 4, "beta")].data_ptr(),
                            act.data_ptr(), self.k16, Mp, M, D, st)
                 self._tc_conv(L[f"ff1{l}"], act, 0, cs, 0, g, (0, cs, 8), 1, 1, M, geglu=1)
                 self._tc_conv(L[f"ff2{l}"], g, 0, cs, 0, h, rm(D), 0, 1, M, res=h, res_strides=rm(D), beta=1.0)
             else:
+                q, k, v = (self.buf(f"bb_{nm}", (B, H, N, Dh), zero=False) for nm in ("q", "k", "v"))
+                self._call("fh_qknorm_rope_f32", qkv.data_ptr(), sd[p + "3.q_norm.gamma"].data_ptr(),
+                           sd[p + "3.k_norm.gamma"].data_ptr(), sd[FH + "transformer.rotary_emb.inv_freq"].data_ptr(),
+                           q.data_ptr(), k.data_ptr(), v.data_ptr(), B, N, H, Dh, st)
                 o = self.buf("bb_o", (M, D), zero=False)
-                self._call("fh_attention_f32", q.data_ptr(), k.data_ptr(), v.data_ptr(), o.data_ptr(), 0, 0, B, H, N, Dh,
+                self._call("fh_attention_f32", q.data_ptr(), k.data_ptr(), v.data_ptr(), o.data_ptr(), B, H, N, Dh,
                            float(b.qk_norm_scale), st)
                 self._sgemm(o, D, sd[p + "3.to_out.weight"], D, None, h, D, 1.0, 1.0, h, D, M, D, D)
                 f = self.buf("bb_a", (M, D), zero=False)
@@ -628,7 +612,7 @@ class Engine:
                 self._sgemm(f, D, sd[p + "5.0.weight"], D, sd[p + "5.0.bias"], None, 0, 0.0, 1.0, u, 2 * self.inner, M,
                             2 * self.inner, D)
                 gg = self.buf("bb_gg", (M, self.inner), zero=False)
-                self._call("fh_geglu_f32", u.data_ptr(), gg.data_ptr(), 0, 0, M, self.inner, self.inner, st)
+                self._call("fh_geglu_f32", u.data_ptr(), gg.data_ptr(), M, self.inner, st)
                 self._sgemm(gg, self.inner, sd[p + "5.3.weight"], self.inner, sd[p + "5.3.bias"], h, D, 1.0, 1.0, h, D, M,
                             D, self.inner)
         gam = sd[FH + "transformer.final_norm.gamma"]
@@ -664,7 +648,7 @@ class Engine:
                 self._call("fh_layernorm_f32", y.data_ptr(), tcnd[(i, "scale")].data_ptr(), tcnd[(i, "shift")].data_ptr(),
                            a.data_ptr(), 0, 0, M, D, 1e-6, st)
                 self._sgemm(a, D, sd[p + "pwconv1.weight"], D, sd[p + "pwconv1.bias"], None, 0, 0.0, 1.0, u, I, M, I, D)
-                self._call("fh_gelu_f32", u.data_ptr(), u.data_ptr(), 0, 0, M, I, st)
+                self._call("fh_gelu_f32", u.data_ptr(), u.data_ptr(), M, I, st)
                 w2, b2 = self.cn_f32[i]  # layer scale folded into pwconv2 at load time
                 self._sgemm(u, I, w2, I, b2, h, D, 1.0, 1.0, h, D, M, D, I)
 

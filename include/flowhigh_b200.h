@@ -39,7 +39,7 @@ int64_t fh_launch_count(void);
 /* Overflow / NaN guard of the 16-bit tensor path.  `status` is a DEVICE uint32 the caller owns and zeroes (NULL turns
  * the guard off); it is remembered per host thread and handed to every later launch from that thread of a kernel that
  * writes 16-bit operands (fh_tc_conv, fh_snake_aa_chunked[_h], fh_to_chunked_16, fh_rmsnorm_f32, fh_layernorm_f32,
- * fh_gelu_f32, fh_geglu_f32, fh_attention_*, fh_qknorm_rope_split, fh_cast_f32_16, fh_sum_cast_f32).  fp16 conversions
+ * fh_qknorm_rope_tiles, fh_attention_tc5, fh_cast_f32_16, fh_sum_cast_f32).  fp16 conversions
  * saturate at +-65504; a saturated, infinite or NaN operand ORs bit 0 into *status.  The host reads the word once per
  * generate() -- the device-side replacement of the reference's per-NFE `torch.isnan(x).any()` prints
  * (models/flow.py:256-267), without their four host syncs per NFE. */
@@ -117,11 +117,11 @@ int fh_dwconv_gelu_res_f32(const float* E, const float* w, const float* b, float
  * fh_dwconv_f32: depthwise Conv1d over time, odd k (7 in ConvNeXtBlock), zero padding, + bias; [B,N,C] fp32, out of place.
  * fh_layernorm_f32: F.layer_norm(x, eps) * w + b per row (AdaLayerNorm with w = scale(t), b = shift(t); b may be NULL);
  *   out_mode as in fh_rmsnorm_f32.
- * fh_gelu_f32: exact-erf GELU, fp32 row-major in, out_mode as in fh_rmsnorm_f32. */
+ * fh_gelu_f32: exact-erf GELU, fp32 row-major in and out. */
 int fh_dwconv_f32(const float* x, const float* w, const float* b, float* out, int B, int N, int C, int k, void* stream);
 int fh_layernorm_f32(const float* x, const float* w, const float* b, void* out, int out_mode, int64_t out_rows,
                      int M, int C, float eps, void* stream);
-int fh_gelu_f32(const float* x, void* out, int out_mode, int64_t out_rows, int M, int C, void* stream);
+int fh_gelu_f32(const float* x, float* out, int M, int C, void* stream);
 
 /* out = x / max(||x||,1e-12) * sqrt(C) * gamma + beta (beta may be NULL)   transformer.py:49-59,82-88
  * out_mode 0: fp32 row-major [M,C];  1: bf16 chunked [C/8][Mp][8] (row pitch out_rows);  2: fp16 chunked. */
@@ -131,33 +131,24 @@ int fh_rmsnorm_f32(const float* x, const float* gamma, const float* beta, void* 
  * attend.py:144-151,179-184; pos_emb.py:45-60 */
 int fh_qknorm_rope_f32(const float* qkv, const float* qg, const float* kg, const float* inv_freq,
                        float* q, float* k, float* v, int B, int N, int H, int D, void* stream);
-/* out[B*N, H*D] = softmax(scale q k^T) v   attend.py:123-137 (no mask)
- * out_mode as in fh_rmsnorm_f32. */
-int fh_attention_f32(const float* q, const float* k, const float* v, void* out, int out_mode,
-                     int64_t out_rows, int B, int H, int N, int D, float scale, void* stream);
-/* 16-bit tensor path of the two calls above.  fh_qknorm_rope_split writes q (pre-multiplied by `scale`) and
- * k as hi + lo 16-bit pairs and v as 16-bit, all [B,H,N,D]; fh_attention_tc computes
- * softmax(qh.kh + ql.kh + qh.kl) v with mma.sync tensor-core tiles (logits reach +-640, see attention_tc.cu). */
-int fh_qknorm_rope_split(const float* qkv, const float* qg, const float* kg, const float* inv_freq,
-                         void* qh, void* ql, void* kh, void* kl, void* v16,
-                         int B, int N, int H, int D, float scale, int fp16, void* stream);
-int fh_attention_tc(const void* qh, const void* ql, const void* kh, const void* kl, const void* v16, void* out,
-                    int out_mode, int64_t out_rows, int B, int H, int N, int D, int fp16, void* stream);
-/* tcgen05 / TMEM form of the same attention (attention_tc5.cu; the default 16-bit path).  fh_qknorm_rope_tiles writes the
- * operands as ready-made shared-memory images of the MMAs (no-swizzle K-major core matrices), one contiguous tile per
- * 128-query tile / 64-key block:
+/* out[B*N, H*D] fp32 row-major = softmax(scale q k^T) v   attend.py:123-137 (no mask) */
+int fh_attention_f32(const float* q, const float* k, const float* v, float* out, int B, int H, int N, int D, float scale,
+                     void* stream);
+/* 16-bit tensor path of the two calls above (attention_tc5.cu): the logits reach +-640, so q (pre-multiplied by `scale`)
+ * and k are hi + lo 16-bit pairs and the logits are S = qh.kh + ql.kh + qh.kl in fp32; v and P are 16-bit.
+ * fh_qknorm_rope_tiles writes the operands as ready-made shared-memory images of the MMAs (no-swizzle K-major core
+ * matrices), one contiguous tile per 128-query tile / 64-key block:
  *   q5 [B*H][ceil(N/128)][hi | lo][D/8][128][8]   k5 [B*H][ceil(N/64)][hi | lo][D/8][64][8]   v5 [B*H][ceil(N/64)][8][D][8]
  * (v5 = V^T, keys past N zero-filled); fh_attention_tc5_operand_elems(which = 0 / 1 / 2, ...) gives their sizes in 16-bit
- * elements.  fh_attention_tc5: S = qh.kh + ql.kh + qh.kl and P.V as tcgen05.mma into TMEM, softmax by one thread per
- * query row, running output in registers; out / out_mode / out_rows as in fh_attention_f32. */
+ * elements.  fh_attention_tc5: S and P.V as tcgen05.mma into TMEM, softmax by one thread per query row, running output
+ * in registers; out [B*N, H*D], out_mode / out_rows as in fh_rmsnorm_f32. */
 int64_t fh_attention_tc5_operand_elems(int which, int B, int H, int N);
 int fh_qknorm_rope_tiles(const float* qkv, const float* qg, const float* kg, const float* inv_freq,
                          void* q5, void* k5, void* v5, int B, int N, int H, int D, float scale, int fp16, void* stream);
 int fh_attention_tc5(const void* q5, const void* k5, const void* v5, void* out, int out_mode, int64_t out_rows,
                      int B, int H, int N, int D, int fp16, void* stream);
 /* g[M,inner] = gelu(u[M, inner + i]) * u[M, i]    transformer.py:92-95 */
-int fh_geglu_f32(const float* u, void* g, int out_mode, int64_t out_rows, int M, int inner, int inner_pad,
-                 void* stream);
+int fh_geglu_f32(const float* u, float* g, int M, int inner, void* stream);
 /* y = a*x + b*z  elementwise (prior: y0 = cond + sigma*eps, cfm_superresolution.py:222-230) */
 int fh_axpby_f32(const float* x, const float* z, float a, float b, float* y, int64_t n, void* stream);
 

@@ -477,42 +477,24 @@ def test_sample_variants_f32(cuda_device, variant):
     assert err <= 3 * floor + 1e-4
 
 
-@pytest.mark.parametrize("precision", ["fp16", "bf16"])
-@pytest.mark.parametrize("N", [51, 128, 333])
-def test_attention_tc_matches_fp32_attention(cuda_device, precision, N):
-    """mma.sync split-operand attention against the fp32 CUDA-core attention on the same q/k/v."""
-    eng, sd, vcfg, g = engine("gen_basic_midpoint", precision)
-    torch.manual_seed(N)
-    B, H, D = 2, 16, 64
-    qkv = torch.randn(B * N, 3 * H * D, device="cuda:0")
-    qg = (1 + 0.1 * torch.randn(H, 1, D, device="cuda:0")).contiguous()
-    kg = (1 + 0.1 * torch.randn(H, 1, D, device="cuda:0")).contiguous()
-    inv_freq = eng.sd["flowhigh.transformer.rotary_emb.inv_freq"]
-    q, k, v = (torch.empty(B, H, N, D, device="cuda:0") for _ in range(3))
-    ref = torch.empty(B * N, H * D, device="cuda:0")
-    eng._call("fh_qknorm_rope_f32", qkv.data_ptr(), qg.data_ptr(), kg.data_ptr(), inv_freq.data_ptr(), q.data_ptr(),
-              k.data_ptr(), v.data_ptr(), B, N, H, D, eng.stream)
-    eng._call("fh_attention_f32", q.data_ptr(), k.data_ptr(), v.data_ptr(), ref.data_ptr(), 0, 0, B, H, N, D, 10.0, eng.stream)
-    s16 = [torch.empty(B, H, N, D, device="cuda:0", dtype=eng.h16) for _ in range(5)]
-    out = torch.empty(B * N, H * D, device="cuda:0")
-    eng._call("fh_qknorm_rope_split", qkv.data_ptr(), qg.data_ptr(), kg.data_ptr(), inv_freq.data_ptr(),
-              *[t.data_ptr() for t in s16], B, N, H, D, 10.0, eng.fp16, eng.stream)
-    eng._call("fh_attention_tc", *[t.data_ptr() for t in s16], out.data_ptr(), 0, 0, B, H, N, D, eng.fp16, eng.stream)
-    torch.cuda.synchronize()
-    # the split reproduces q, k to ~2^-21 (fp16) / 2^-16 (bf16): logits agree to 1e-3; the remaining error is the
-    # 16-bit rounding of P and V in the P.V product
-    err = float((out - ref).abs().max())
-    rel = float((out - ref).norm() / ref.norm())
-    print(f"attention_tc {precision} N={N}: max-abs {err:.3g}, rel-L2 {rel:.3g}")
-    assert rel <= (2e-3 if precision == "fp16" else 1e-2)
+# rel-L2 against the fp32 attention of the mma.sync split-operand kernel (same arithmetic as tcgen05: split logits, 16-bit
+# P; a different summation order), on the seeded inputs of the test below.  That kernel measured 2.9 x slower and was
+# removed; these are its values, printed to full precision on a B200 at commit 37e0ca4.
+MMA_SYNC_ATTENTION_REL = {
+    ("fp16", 1): 2.113479131e-04, ("fp16", 51): 2.096002572e-04, ("fp16", 64): 2.091491042e-04, ("fp16", 128): 2.087157045e-04,
+    ("fp16", 129): 2.083572181e-04, ("fp16", 333): 2.087086759e-04, ("fp16", 1000): 2.080944687e-04,
+    ("bf16", 1): 1.661566901e-03, ("bf16", 51): 1.665844466e-03, ("bf16", 64): 1.671219128e-03, ("bf16", 128): 1.667293138e-03,
+    ("bf16", 129): 1.670291997e-03, ("bf16", 333): 1.662420458e-03, ("bf16", 1000): 1.663677278e-03,
+}
 
 
 @pytest.mark.parametrize("precision", ["fp16", "bf16"])
 @pytest.mark.parametrize("N", [1, 51, 64, 128, 129, 333, 1000])
-def test_attention_tc5_matches_fp32_attention(cuda_device, precision, N):
-    """tcgen05 / TMEM attention (the default 16-bit path) against the fp32 CUDA-core attention on the same q/k/v: every
+def test_attention_tc5_matches_fp32_attention_pinned(cuda_device, precision, N):
+    """tcgen05 / TMEM attention (the 16-bit path) against the fp32 CUDA-core attention on the same q/k/v: every
     tile-boundary case (one key, a partial key block, exactly one / two blocks, a partial query tile, the N = 1000 of the
-    timed configuration), the chunked 16-bit output the backbone consumes, and stale operand buffers from a longer call."""
+    timed configuration), the chunked 16-bit output the backbone consumes, and stale operand buffers from a longer call;
+    the rel-L2 also stays within 1.5 x of the removed mma.sync kernel's, pinned per case in MMA_SYNC_ATTENTION_REL."""
     eng, sd, vcfg, g = engine("gen_basic_midpoint", precision)
     torch.manual_seed(N)
     B, H, D = 2, 16, 64
@@ -524,7 +506,7 @@ def test_attention_tc5_matches_fp32_attention(cuda_device, precision, N):
     ref = torch.empty(B * N, H * D, device="cuda:0")
     eng._call("fh_qknorm_rope_f32", qkv.data_ptr(), qg.data_ptr(), kg.data_ptr(), inv_freq.data_ptr(), q.data_ptr(),
               k.data_ptr(), v.data_ptr(), B, N, H, D, eng.stream)
-    eng._call("fh_attention_f32", q.data_ptr(), k.data_ptr(), v.data_ptr(), ref.data_ptr(), 0, 0, B, H, N, D, 10.0, eng.stream)
+    eng._call("fh_attention_f32", q.data_ptr(), k.data_ptr(), v.data_ptr(), ref.data_ptr(), B, H, N, D, 10.0, eng.stream)
     # operand buffers pre-filled with NaN bit patterns: rows / keys past N must never reach a kept output
     ops = [torch.full((int(eng.lib.fh_attention_tc5_operand_elems(w, B, H, N)),), float("nan"), device="cuda:0", dtype=eng.h16)
            for w in range(3)]
@@ -536,13 +518,7 @@ def test_attention_tc5_matches_fp32_attention(cuda_device, precision, N):
     assert torch.isfinite(out).all()
     err = float((out - ref).abs().max())
     rel = float((out - ref).norm() / ref.norm())
-    # the mma.sync kernel on the same inputs: same arithmetic (split logits, 16-bit P), different summation order
-    s16 = [torch.empty(B, H, N, D, device="cuda:0", dtype=eng.h16) for _ in range(5)]
-    old = torch.empty(B * N, H * D, device="cuda:0")
-    eng._call("fh_qknorm_rope_split", qkv.data_ptr(), qg.data_ptr(), kg.data_ptr(), inv_freq.data_ptr(),
-              *[t.data_ptr() for t in s16], B, N, H, D, 10.0, eng.fp16, eng.stream)
-    eng._call("fh_attention_tc", *[t.data_ptr() for t in s16], old.data_ptr(), 0, 0, B, H, N, D, eng.fp16, eng.stream)
-    rel_old = float((old - ref).norm() / ref.norm())
+    rel_old = MMA_SYNC_ATTENTION_REL[(precision, N)]
     print(f"attention_tc5 {precision} N={N}: max-abs {err:.3g}, rel-L2 {rel:.3g} (mma.sync kernel: {rel_old:.3g})")
     assert rel <= (2e-3 if precision == "fp16" else 1e-2)
     assert rel <= 1.5 * rel_old + 1e-4

@@ -3,7 +3,7 @@
 name=$1; shift
 cd "$(dirname "$0")/../flowhigh_b200" || exit 1
 mkdir -p lib/obj_$name
-for f in dsp backbone vocoder_f32 vocoder_tc tc_conv attention_tc attention_tc5; do
+for f in dsp backbone vocoder_f32 vocoder_tc tc_conv attention_tc5; do
   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 -Xcompiler -fPIC -Xcompiler -fvisibility=hidden "$@" \
     -c csrc/$f.cu -o lib/obj_$name/$f.o &
 done

@@ -5,7 +5,7 @@ rows = list(csv.reader(open(sys.argv[1])))
 h = [i for i, r in enumerate(rows) if r and r[0] == "ID"][0]
 H = rows[h]
 ki, mi, ui, vi = H.index("Kernel Name"), H.index("Metric Name"), H.index("Metric Unit"), H.index("Metric Value")
-fam = {"tc_conv_kernel": "tc_conv", "tc_conv2_kernel": "tc_conv", "snake_aa": "snake", "attention_tc": "attention"}
+fam = {"tc_conv_kernel": "tc_conv", "tc_conv2_kernel": "tc_conv", "snake_aa": "snake", "attention_tc5": "attention"}
 agg = collections.defaultdict(lambda: {"launches": 0, "dram_read_bytes": 0.0, "dram_write_bytes": 0.0, "ncu_ms": 0.0})
 scale = {"byte": 1.0, "Kbyte": 1e3, "Mbyte": 1e6, "Gbyte": 1e9, "ns": 1e-6, "us": 1e-3, "ms": 1.0, "s": 1e3}
 for r in rows[h + 1:]:

@@ -21,7 +21,7 @@ from os import environ as _environ
 _os_environ_get = _environ.get
 import ctypes as C
 import math
-from typing import Dict, Optional
+from typing import Dict, Optional, Sequence, Tuple
 
 import numpy as np
 import torch
@@ -372,27 +372,52 @@ class Engine:
         """x [B, T_in] fp32 on device -> cond [B, T] = resample(x) / max|.|: `method='scipy'` is
         scipy.signal.resample_poly's filter (flowhighsr.py:68-69), `'soxr_hq'` the filter of the librosa branch
         (flowhighsr.py:74-80; tables.resample_plan_soxr_hq) -- same polyphase kernel, different taps."""
-        self._chk(x)
-        B, T_in = x.shape
+        return self.resample_normalise_parts([(x, sr_in)], sr_out, method)
+
+    def resample_normalise_parts(self, parts: Sequence[Tuple[torch.Tensor, int]], sr_out: int = 48000,
+                                 method: str = "scipy") -> torch.Tensor:
+        """Clips of several input rates with one output length in one batch: parts [(x_r [B_r, T_r], sr_r)] ->
+        cond [sum B_r, T_out], rows in part order, each row exactly what `resample_normalise` gives for it alone.  One
+        resampler launch per part into its rows of the shared buffer (a 48 kHz part is copied there), then one
+        normalisation launch for the whole batch."""
+        for x, _ in parts:
+            self._chk(x)
         if method not in ("scipy", "soxr_hq"):
             raise ValueError(f"unknown resampling method {method!r} (scipy|soxr_hq)")
-        plan = tables.resample_plan(sr_in, sr_out) if method == "scipy" else tables.resample_plan_soxr_hq(sr_in, sr_out)
+        if not parts:
+            raise ValueError("resample_normalise_parts needs at least one part")
+        plans, T_out = [], None
+        for x, sr_in in parts:
+            plan = tables.resample_plan(sr_in, sr_out) if method == "scipy" else tables.resample_plan_soxr_hq(sr_in, sr_out)
+            n = x.shape[1] if plan is None else tables.resample_out_len(x.shape[1], plan[1], plan[2])
+            if T_out is not None and n != T_out:
+                raise ValueError(f"parts resample to different lengths ({T_out} and {n} samples)")
+            plans.append(plan)
+            T_out = n
+        B = sum(x.shape[0] for x, _ in parts)
         absmax = self.buf("rs_absmax", (B,), torch.int32)
         self._call("fh_fill_u32", absmax.data_ptr(), 0, B, self.stream)
-        if plan is None:
-            y, T_out = x, T_in
+        if len(parts) == 1 and plans[0] is None:  # 48 kHz in, one part: normalised straight from the input
+            y = parts[0][0]
             self._call("fh_absmax_f32", y.data_ptr(), absmax.data_ptr(), B, T_out, self.stream)
         else:
-            h, up, down, npp, npr = plan
-            key = (sr_in, sr_out, method)
-            if key not in self._resample_taps:
-                self._resample_taps[key] = torch.from_numpy(h).to(self.device)
-            hd = self._resample_taps[key]
-            T_out = tables.resample_out_len(T_in, up, down)
             y = self.buf("rs_y", (B, T_out), zero=False)
-            self._call("fh_resample_poly_f32", x.data_ptr(), y.data_ptr(), hd.data_ptr(), absmax.data_ptr(), B, T_in,
-                       T_out, hd.numel(), up, down, npp, npr, self.stream,
-                       work={"bytes": 4.0 * B * (T_in + T_out), "flops": 2.0 * B * T_out * (hd.numel() // up + 1)})
+            r0 = 0
+            for (x, sr_in), plan in zip(parts, plans):
+                B_r, T_in = x.shape
+                if plan is None:
+                    y[r0: r0 + B_r].copy_(x)
+                    self._call("fh_absmax_f32", y[r0:].data_ptr(), absmax[r0:].data_ptr(), B_r, T_out, self.stream)
+                else:
+                    h, up, down, npp, npr = plan
+                    key = (sr_in, sr_out, method)
+                    if key not in self._resample_taps:
+                        self._resample_taps[key] = torch.from_numpy(h).to(self.device)
+                    hd = self._resample_taps[key]
+                    self._call("fh_resample_poly_f32", x.data_ptr(), y[r0:].data_ptr(), hd.data_ptr(), absmax[r0:].data_ptr(),
+                               B_r, T_in, T_out, hd.numel(), up, down, npp, npr, self.stream,
+                               work={"bytes": 4.0 * B_r * (T_in + T_out), "flops": 2.0 * B_r * T_out * (hd.numel() // up + 1)})
+                r0 += B_r
         cond = torch.empty((B, T_out), dtype=torch.float32, device=self.device)
         self._call("fh_scale_by_absmax_f32", y.data_ptr(), cond.data_ptr(), absmax.data_ptr(), 1.0, B, T_out, self.stream,
                    work={"bytes": 8.0 * B * T_out})

@@ -17,6 +17,7 @@ from __future__ import annotations
 
 import collections
 import json
+import math
 from pathlib import Path
 from typing import Dict, List, Optional, Sequence, Union
 
@@ -24,6 +25,7 @@ import numpy as np
 import torch
 from torch import nn
 
+from . import tables
 from .config import BackboneConfig, CFM_METHODS, VocoderConfig
 from .engine import Engine
 from .weights import FH, VOC, fold_weight_norm, random_state_dict, state_dict_spec
@@ -67,6 +69,20 @@ class _Tree(nn.Module):
 
 def _is_buffer(key: str) -> bool:
     return key.endswith(".filter") or key.endswith("inv_freq")
+
+
+def group_by_output_length(lengths: Sequence[int], srs: Sequence[int], target_sr: int, method: str) -> Dict[tuple, List[int]]:
+    """Clip indices of one batched call -> {(T_out, method): indices}.  Only the resampler depends on the input rate: every
+    kernel behind it sees [B, T_out] rows, so clips of one output length (`tables.resample_out_len`; the input length
+    when the input is already at `target_sr`) share one batch whatever their rate and input length.  Inside a group the
+    clips of one (rate, input length) part are consecutive, because the resampler runs one launch per part over
+    contiguous rows: parts in the order of their first clip, clips of a part in caller order."""
+    groups: Dict[tuple, Dict[tuple, List[int]]] = {}
+    for i, (n, s) in enumerate(zip(lengths, srs)):
+        g = math.gcd(int(target_sr), int(s))
+        T_out = tables.resample_out_len(int(n), int(target_sr) // g, int(s) // g)
+        groups.setdefault((T_out, method), {}).setdefault((int(s), int(n)), []).append(i)
+    return {key: [i for idxs in parts.values() for i in idxs] for key, parts in groups.items()}
 
 
 class MelVoco(_Tree):
@@ -281,21 +297,22 @@ class FlowHighSR(nn.Module):
             return None
         return dict(tableau=self._tableau, atol=float(self.odeint_kwargs["atol"]), rtol=float(self.odeint_kwargs["rtol"]))
 
-    def _staging(self, B: int, n: int) -> torch.Tensor:
-        """Page-locked [B, n] fp32 staging buffer of the batched host path, cached per shape (a few entries, least recently
-        used out).  The previous upload from it must have left the host before it is refilled."""
+    def _staging(self, numel: int) -> torch.Tensor:
+        """Page-locked flat fp32 staging buffer of the batched host path (the clips of a group one after the other), cached
+        per size (a few entries, least recently used out).  The previous upload from it must have left the host before it
+        is refilled."""
         if getattr(self, "_stage_event", None) is None:
             self._stage_event = torch.cuda.Event()
             self._stage_bufs = collections.OrderedDict()
         else:
             self._stage_event.synchronize()
-        buf = self._stage_bufs.get((B, n))
+        buf = self._stage_bufs.get(numel)
         if buf is None:
-            buf = self._stage_bufs[(B, n)] = torch.empty((B, n), dtype=torch.float32).pin_memory()
+            buf = self._stage_bufs[numel] = torch.empty(numel, dtype=torch.float32).pin_memory()
             while len(self._stage_bufs) > 4:
                 self._stage_bufs.popitem(last=False)
         else:
-            self._stage_bufs.move_to_end((B, n))
+            self._stage_bufs.move_to_end(numel)
         return buf
 
     def _resample_method(self) -> str:
@@ -376,29 +393,31 @@ class FlowHighSR(nn.Module):
                        out_host: Optional[torch.Tensor] = None) -> List[torch.Tensor]:
         """Batched `generate`: every clip is processed exactly as the reference processes it alone
         (per-clip peak normalisation, attention, cutoff and output normalisation; SURVEY.md F8).
-        Clips sharing (sr, length) run as one batch through every kernel.
+        Clips with the same OUTPUT length run as one batch through every kernel, whatever their input rates and input
+        lengths (`group_by_output_length`): the resampler runs once per (rate, input length) part of the batch, everything
+        behind it once for the whole batch.  Clips of different output lengths run as separate batches; the results come
+        back in caller order either way.
 
         `out_host` (optional, page-locked `[n_clips, T]` fp32): every result is ALSO copied there, asynchronously, on a
         side stream; groups of >= 2 * `overlap_min_batch` clips (off by default, see __init__) run as two sub-batches so
         that the device -> host copy of the first overlaps the kernels of the second (the output of a 64 x 10 s batch is
         123 MB, ~5 ms of PCIe time).  The caller synchronises the device (or `self.copy_stream`) before reading `out_host`."""
-        self._resample_method()
+        method = self._resample_method()
         eng = self._engine()
         eng.new_call()
-        srs = [sr] * len(audios) if isinstance(sr, int) else list(sr)
+        srs = [int(s) for s in ([sr] * len(audios) if isinstance(sr, int) else sr)]
         # grouping needs the lengths only; the per-clip preparation (int16 heuristic = a pass over the samples, fp32 copy)
         # runs sub-batch by sub-batch below, so the host work of sub-batch k + 1 hides behind the kernels of sub-batch k
         prepped: List[Optional[np.ndarray]] = [None] * len(audios)
-        groups: Dict[tuple, List[int]] = {}
-        for i, (a, s) in enumerate(zip(audios, srs)):
-            groups.setdefault((int(s), self._clip_len(a)), []).append(i)
+        lens = [self._clip_len(a) for a in audios]
+        groups = group_by_output_length(lens, srs, int(target_sampling_rate), method)
         if out_host is not None:
             if not (out_host.is_pinned() and out_host.dtype == torch.float32 and out_host.dim() == 2
                     and out_host.shape[0] >= len(audios) and out_host.is_contiguous()):
                 raise ValueError("out_host must be a contiguous page-locked fp32 tensor [n_clips, T]")
             if getattr(self, "copy_stream", None) is None:
                 self.copy_stream = torch.cuda.Stream(eng.device)
-            # sub-batches: [(rate, length), clip indices]
+            # sub-batches: [(output length, method), clip indices]
             work = []
             for key, idxs in groups.items():
                 if len(idxs) >= 2 * self.overlap_min_batch:
@@ -412,7 +431,7 @@ class FlowHighSR(nn.Module):
         flags = 0
         check = self.overflow_check != "off" and eng.tc
         main = torch.cuda.current_stream(eng.device)
-        for gi, ((s, n), idxs) in enumerate(work):
+        for gi, ((T_out, _), idxs) in enumerate(work):
             if check and gi > 0 and out_host is None:
                 flags |= eng.status_read()  # one status word per engine: collect the previous group's before the next resets it
             graphed = self.cuda_graphs and len(idxs) <= self.cuda_graph_max_batch and not self.use_torchode
@@ -425,21 +444,24 @@ class FlowHighSR(nn.Module):
             pinned_done = False
             # with out_host the status word is reset once and accumulates over all sub-batches (no host sync in between)
             reset = out_host is None or gi == 0
+            # the clips' samples one after the other, in `idxs` order: part r is a [count_r, n_r] block of it
+            parts = self._parts(idxs, srs, lens)
+            offs = np.cumsum([0] + [lens[i] for i in idxs]).tolist()
             if direct:
-                x = torch.empty((len(idxs), n), dtype=torch.float32, device=eng.device)
+                x = torch.empty(offs[-1], dtype=torch.float32, device=eng.device)
                 for j, i in enumerate(idxs):
-                    x[j].copy_(audios[i].reshape(-1), non_blocking=True)
+                    x[offs[j]: offs[j + 1]].copy_(audios[i].reshape(-1), non_blocking=True)
                 host = None
             else:
                 for i in idxs:
                     prepped[i] = self._prep_input(audios[i])
                 if pinned:  # one copy per clip into a cached page-locked staging buffer (no np.stack, no fresh cudaHostAlloc)
-                    host = self._staging(len(idxs), n)
+                    host = self._staging(offs[-1])
                     view = host.numpy()
                     for j, i in enumerate(idxs):
-                        view[j] = prepped[i]
+                        view[offs[j]: offs[j + 1]] = prepped[i]
                 else:
-                    host = torch.from_numpy(np.stack([prepped[i] for i in idxs]))
+                    host = torch.from_numpy(np.concatenate([prepped[i] for i in idxs]))
 
             def read_back(first, chunk):  # results of clips idxs[first : first + len(chunk)] -> out_host, on the copy stream
                 if chunk.shape[1] > out_host.shape[1]:
@@ -460,7 +482,7 @@ class FlowHighSR(nn.Module):
 
             chunked = False
             if graphed and reset:
-                outs = [self._run_group_graphed(eng, host, s, int(target_sampling_rate), int(timestep), e)]
+                outs = [self._run_group_graphed(eng, host, parts, T_out, int(target_sampling_rate), int(timestep), e)]
             else:
                 if not direct:
                     x = host.to(eng.device, non_blocking=True)
@@ -469,7 +491,7 @@ class FlowHighSR(nn.Module):
                 # large batches with a host destination: post-processing in chunks of `readback_chunk` clips, so that the
                 # device -> host copy of a chunk overlaps the post-processing of the next (only the last chunk's copy is exposed)
                 chunked = out_host is not None and self.readback_chunk and len(idxs) >= 2 * self.readback_chunk
-                outs = self._run_group(eng, x, s, int(target_sampling_rate), int(timestep),
+                outs = self._run_group(eng, self._split(x, parts), int(target_sampling_rate), int(timestep),
                                        None if e is None else e.to(eng.device), reset_status=reset,
                                        pp_chunk=self.readback_chunk if chunked else 0, on_chunk=read_back if chunked else None)
                 if not chunked:
@@ -488,13 +510,34 @@ class FlowHighSR(nn.Module):
             self._check_status(eng, flags | eng.status_read())
         return results  # type: ignore[return-value]
 
-    def _run_group(self, eng, x, sr, target_sr, timestep, eps_dev, reset_status: bool = True, pp_chunk: int = 0, on_chunk=None):
-        """resample -> log-mel -> CFM -> vocoder -> post-processing for one batch of equal-length clips.
+    @staticmethod
+    def _parts(idxs: Sequence[int], srs: Sequence[int], lens: Sequence[int]) -> List[tuple]:
+        """(rate, input length, count) of every run of consecutive clips of one rate and length in `idxs`."""
+        parts: List[list] = []
+        for i in idxs:
+            if parts and parts[-1][:2] == [srs[i], lens[i]]:
+                parts[-1][2] += 1
+            else:
+                parts.append([srs[i], lens[i], 1])
+        return [tuple(p) for p in parts]
+
+    @staticmethod
+    def _split(x: torch.Tensor, parts: Sequence[tuple]) -> List[tuple]:
+        """Flat device samples of a group -> [(x_r [count, n] view, rate)] per part."""
+        out, o = [], 0
+        for s, n, c in parts:
+            out.append((x[o: o + c * n].view(c, n), s))
+            o += c * n
+        return out
+
+    def _run_group(self, eng, parts, target_sr, timestep, eps_dev, reset_status: bool = True, pp_chunk: int = 0, on_chunk=None):
+        """resample -> log-mel -> CFM -> vocoder -> post-processing for one batch of clips of one output length, given as
+        parts [(x_r [count, n] on the device, rate)].
         `pp_chunk` > 0: the post-processing (per clip anyway) runs in chunks of that many clips, `on_chunk(first, out)` is
         called after each (the caller starts its device -> host copy there), and the list of chunk results is returned."""
         if reset_status:
             eng.status_begin()
-        cond = eng.resample_normalise(x, sr, target_sr, method=self._resample_method())
+        cond = eng.resample_normalise_parts(parts, target_sr, method=self._resample_method())
         cond_mel = eng.encode(cond)
         mel = eng.sample_mel(cond_mel, self._noise_like(cond_mel, eps_dev), steps=timestep,
                              ode_method=self.odeint_kwargs["method"], cfm_method=self.cfm_method, sigma=float(self.sigma),
@@ -533,13 +576,15 @@ class FlowHighSR(nn.Module):
                 f"flowhigh_b200: a {eng.precision} tensor-core operand overflowed or was not finite (status {flags:#x}); "
                 "the result is not trustworthy -- use precision='bf16' (fp32 range) or 'fp32' for these weights / inputs")
 
-    def _run_group_graphed(self, eng, host, sr, target_sr, timestep, eps_host):
+    def _run_group_graphed(self, eng, host, parts, T, target_sr, timestep, eps_host):
         """Small batches are launch-bound (~300 kernel launches per clip): the whole per-shape pipeline is captured
-        into a CUDA graph (static input / noise / output buffers) and replayed.  A shape is captured when it is seen
-        for the `cuda_graph_min_hits`-th time; the cache holds `cuda_graph_cache_size` graphs, least recently used out
-        (each entry owns its static buffers, its private pool and references to the engine buffers it replays into)."""
-        B, n = host.shape
-        key = (B, n, sr, target_sr, timestep, self.odeint_kwargs["method"], self.cfm_method, float(self.sigma),
+        into a CUDA graph (static input / noise / output buffers) and replayed.  `host` holds the group's samples flat,
+        `parts` its ordered (rate, input length, count) parts, `T` its output length; a shape is that tuple of parts.
+        A shape is captured when it is seen for the `cuda_graph_min_hits`-th time; the cache holds
+        `cuda_graph_cache_size` graphs, least recently used out (each entry owns its static buffers, its private pool and
+        references to the engine buffers it replays into)."""
+        B = sum(c for _, _, c in parts)
+        key = (tuple(parts), target_sr, timestep, self.odeint_kwargs["method"], self.cfm_method, float(self.sigma),
                self.upsampling_method)
         ent = self._graphs.get(key)
         if ent is None:
@@ -550,23 +595,24 @@ class FlowHighSR(nn.Module):
                 self._graph_seen.popitem(last=False)
             if seen < self.cuda_graph_min_hits:
                 x = host.to(eng.device, non_blocking=True)
-                return self._run_group(eng, x, sr, target_sr, timestep, None if eps_host is None else eps_host.to(eng.device))
-            x_static = torch.zeros((B, n), dtype=torch.float32, device=eng.device)
+                return self._run_group(eng, self._split(x, parts), target_sr, timestep,
+                                       None if eps_host is None else eps_host.to(eng.device))
+            x_static = torch.zeros(host.shape, dtype=torch.float32, device=eng.device)
             x_static.copy_(host)
-            T = -(-n * (target_sr // np.gcd(target_sr, sr)) // (sr // np.gcd(target_sr, sr)))
             eps_static = torch.randn((B, T // 480, 256), dtype=torch.float32, device=eng.device)
+            parts_static = self._split(x_static, parts)
             eng._touch_log = {}
             try:
                 side = torch.cuda.Stream(eng.device)
                 side.wait_stream(torch.cuda.current_stream(eng.device))
                 with torch.cuda.stream(side):
                     for _ in range(2):  # allocate persistent buffers, time-conditioning cache, function attributes
-                        self._run_group(eng, x_static, sr, target_sr, timestep, eps_static)
+                        self._run_group(eng, parts_static, target_sr, timestep, eps_static)
                 torch.cuda.current_stream(eng.device).wait_stream(side)
                 torch.cuda.synchronize(eng.device)
                 graph = torch.cuda.CUDAGraph()
                 with torch.cuda.graph(graph):
-                    out_static = self._run_group(eng, x_static, sr, target_sr, timestep, eps_static)
+                    out_static = self._run_group(eng, parts_static, target_sr, timestep, eps_static)
                 keep = list(eng._touch_log.values())
             finally:
                 eng._touch_log = None
@@ -654,8 +700,9 @@ class FlowHighSR(nn.Module):
                          eps: Optional[Sequence[torch.Tensor]] = None, max_batch: int = 64, group=None, gather: bool = True):
         """A list of clips (mixed input rates allowed, equal OUTPUT length) over the GPUs of one box: every rank calls
         this with the same list, `sharding.assign_clips` gives rank r its clips, they run through `generate_batch` in
-        batches of <= max_batch per (rate, length) group, and -- when `gather` -- ONE all_gather_into_tensor puts the
-        [n_clips, T] fp32 result on every rank in clip order.  No collective on the data path itself."""
+        batches of <= max_batch per output-length group (clips of different input rates share a batch), and -- when
+        `gather` -- ONE all_gather_into_tensor puts the [n_clips, T] fp32 result on every rank in clip order.  No
+        collective on the data path itself."""
         import torch.distributed as dist
         from . import sharding
         distributed = dist.is_available() and dist.is_initialized()
@@ -666,13 +713,13 @@ class FlowHighSR(nn.Module):
         parts = sharding.assign_clips(out_len, world)
         mine = parts[rank]
         results: List[Optional[torch.Tensor]] = [None] * len(mine)
-        by_rate: Dict[tuple, List[int]] = {}
-        for j, i in enumerate(mine):
-            by_rate.setdefault((int(srs[i]), int(np.asarray(audios[i]).shape[-1])), []).append(j)
-        for (s, _n), js in by_rate.items():
+        groups = group_by_output_length([self._clip_len(audios[i]) for i in mine], [int(srs[i]) for i in mine],
+                                        int(target_sampling_rate), self._resample_method())
+        for js in groups.values():
             for b0 in range(0, len(js), max_batch):
                 sel = js[b0: b0 + max_batch]
-                outs = self.generate_batch([audios[mine[j]] for j in sel], s, target_sampling_rate, timestep,
+                outs = self.generate_batch([audios[mine[j]] for j in sel], [int(srs[mine[j]]) for j in sel],
+                                           target_sampling_rate, timestep,
                                            eps=None if eps is None else [eps[mine[j]] for j in sel], pinned=True)
                 for j, o in zip(sel, outs):
                     results[j] = o

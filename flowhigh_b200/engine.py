@@ -26,7 +26,7 @@ from typing import Dict, Optional, Sequence, Tuple
 import numpy as np
 import torch
 
-from . import _lib, packing, tables
+from . import _lib, packing, rk, tables
 from .config import BackboneConfig, MelConfig, VocoderConfig
 from .weights import FH, VOC
 
@@ -780,15 +780,129 @@ class Engine:
             self.ode_stats.append({"n_steps": n_steps, "n_accepted": n_acc, "n_f_evals": nfe})
         return out
 
+    def _rk4_step(self, y, cond, null, t0, t1, cond_scale, packed):
+        """One step of torchdiffeq's `rk4` (rk4_alt_step_func: the 3/8 rule, last stage at the grid point t1), y in place:
+        k1 = f(t0, y), k2 = f(t0 + dt/3, y + dt k1/3), k3 = f(t0 + 2dt/3, y + dt (k2 - k1/3)), k4 = f(t1, y + dt (k1 - k2 + k3)),
+        y += (k1 + 3 (k2 + k3) + k4) dt / 8.  Stage times in fp32 like the reference's fp32 grid; the last NFE writes
+        y + dt (k1 + 3 k2 + 3 k3) / 8 + dt/8 k4 from its to_pred epilogue."""
+        n = y.numel()
+        K = self.buf("rk4_k", (3,) + tuple(y.shape), zero=False)
+        ys = self.buf("rk4_ys", y.shape, zero=False)
+        yb = self.buf("rk4_yb", y.shape, zero=False)
+        zero = self.buf("rk4_zero", y.shape)
+        st = self.stream
+        t0, t1 = np.float32(t0), np.float32(t1)
+        dt = np.float32(t1 - t0)
+        third = float(dt) / 3.0
+
+        def lincomb(coefs, dst):
+            arr = (C.c_float * len(coefs))(*coefs)
+            self._call("fh_rk_lincomb_f32", y.data_ptr(), K.data_ptr(), n, len(coefs), arr, dst.data_ptr(), n, st)
+
+        packed = self._field_update(y, cond, null, float(t0), zero, 1.0, K[0], cond_scale, packed)
+        lincomb([third], ys)
+        packed = self._field_update(ys, cond, null, float(t0 + dt * np.float32(1.0 / 3.0)), zero, 1.0, K[1], cond_scale,
+                                    packed)
+        lincomb([-third, float(dt)], ys)
+        packed = self._field_update(ys, cond, null, float(t0 + dt * np.float32(2.0 / 3.0)), zero, 1.0, K[2], cond_scale,
+                                    packed)
+        lincomb([float(dt), -float(dt), float(dt)], ys)
+        lincomb([0.125 * float(dt), 0.375 * float(dt), 0.375 * float(dt)], yb)
+        return self._field_update(ys, cond, null, float(t1), yb, 0.125 * float(dt), y, cond_scale, packed)
+
+    def _odeint_dopri5(self, y0: torch.Tensor, cond_mel: torch.Tensor, null, cond_scale: float, t0: float, t1: float, *,
+                       atol: float, rtol: float, joint: bool, max_steps: int = 10000) -> torch.Tensor:
+        """y(t1) by torchdiffeq's `dopri5` (cfm_superresolution.py:243 with `torchdiffeq_ode_method='dopri5'`): Dormand-Prince
+        stages with FSAL, Shampine's error estimate, torchdiffeq's controller (`rk.TorchdiffeqController`) and its quartic
+        dense output at t1 from the last accepted step, which ends at or past t1 (the field is evaluated at t > 1 then).
+        torchdiffeq solves whatever tensor it is given as ONE problem: one step sequence, the rms error norm over the
+        whole tensor.  `joint=True` does that for the batch (`sample()` with B > 1); `joint=False` solves every clip on its
+        own (`generate` is batch-1 in the reference, so the `generate*` paths see per-clip step sequences).  Times and
+        controller arithmetic are fp64 on the host, the field gets fp32 times; one 8-byte read per attempted step."""
+        B, N, Din = y0.shape
+        inst = [(0, B)] if joint else [(b, b + 1) for b in range(B)]
+        Bi = inst[0][1] - inst[0][0]
+        n = Bi * N * Din
+        tab = rk.DOPRI5
+        ctl = rk.TorchdiffeqController(atol=float(atol), rtol=float(rtol))
+        out = torch.empty_like(y0)
+        K = self.buf("rk_k", (8, Bi, N, Din), zero=False)   # k_0 .. k_6, slot 7 = scratch (error estimate / f1 - f0)
+        ys = self.buf("rk_ys", (Bi, N, Din), zero=False)
+        zero = self.buf("rk_zero", (Bi, N, Din))
+        ssq = self.buf("rk_ssq", (1,), torch.float64, zero=False)
+        st = self.stream
+        self.ode_stats = []
+        f32 = np.float32
+
+        def lincomb(base, coefs, dst):
+            arr = (C.c_float * len(coefs))(*[float(c) for c in coefs])
+            self._call("fh_rk_lincomb_f32", _ptr(base), K.data_ptr(), n, len(coefs), arr, dst.data_ptr(), n, st)
+
+        def norm(e, ya, yb):
+            self._call("fh_rk_scaled_sumsq_f32", e.data_ptr(), ya.data_ptr(), _ptr(yb), ctl.atol, ctl.rtol, 1, n,
+                       ssq.data_ptr(), st)
+            return float(np.sqrt(ssq.item() / n))
+
+        for b0, b1 in inst:
+            y = out[b0: b1]
+            self._call("fh_axpby_f32", y0[b0: b1].data_ptr(), None, 1.0, 0.0, y.data_ptr(), n, st)
+            cond = cond_mel[b0: b1]
+            nullb = None if null is None else null[b0: b1]
+            packed = False
+
+            def field(x, t, slot):  # K[slot] = v(float32(t), x)
+                nonlocal packed
+                packed = self._field_update(x, cond, nullb, float(f32(t)), zero, 1.0, K[slot], cond_scale, packed)
+
+            t = float(t0)
+            field(y, t, 0)
+            # Hairer's initial step: d0 = |y0|, d1 = |f0|, d2 = |f(t0 + h0, y0 + h0 f0) - f0| / h0 in the scaled rms norm
+            d0, d1 = norm(y, y, None), norm(K[0], y, None)
+            h0 = ctl.initial_dt(d0, d1)
+            lincomb(y, [h0], ys)
+            field(ys, t + h0, 1)
+            lincomb(None, [-1.0, 1.0], K[7])
+            dt = ctl.initial_dt_refine(h0, d1, norm(K[7], y, None) / h0)
+            nfe, n_steps, n_acc = 2, 0, 0
+            while t < t1:
+                if n_steps >= max_steps:
+                    raise RuntimeError(f"adaptive solve did not reach t_end in {max_steps} steps (clip {b0}, t = {t})")
+                # torchdiffeq casts t0, dt and t0 + dt to the state's fp32 for the stages; stages with c = 1 sit at t0 + dt
+                t_end = t + dt
+                t32, dt32 = f32(t), f32(dt)
+                for s in range(1, 7):
+                    lincomb(y, [dt32 * f32(w) for w in tab.a[s]], ys)
+                    field(ys, f32(t_end) if tab.c[s] == 1.0 else t32 + f32(tab.c[s]) * dt32, s)
+                nfe += 6
+                # ys now holds the 5th-order solution (FSAL: the last stage is evaluated at it)
+                lincomb(None, [dt32 * f32(w) for w in rk.DPS_C_ERROR], K[7])
+                ratio = norm(K[7], y, ys)
+                n_steps += 1
+                if ctl.accept(ratio):
+                    n_acc += 1
+                    if t_end >= t1:  # dense output at t1 from (y0, k_0 .. k_6) of this step
+                        x = f32((t1 - t) / (t_end - t))
+                        lincomb(y, rk.dopri5_dense_weights(float(x), float(dt32)), y)
+                        break
+                    t = t_end
+                    self._call("fh_axpby_f32", ys.data_ptr(), None, 1.0, 0.0, y.data_ptr(), n, st)
+                    self._call("fh_axpby_f32", K[6].data_ptr(), None, 1.0, 0.0, K[0].data_ptr(), n, st)
+                dt = ctl.next_dt(dt, ratio)
+            self.ode_stats.append({"n_steps": n_steps, "n_accepted": n_acc, "n_f_evals": nfe})
+        return out
+
     def sample_mel(self, cond_mel: torch.Tensor, eps: torch.Tensor, *, steps: int, ode_method: str, cfm_method: str,
                    sigma: float, cond_scale: float = 1.0, mel_pp: bool = False, std_1: Optional[float] = None,
-                   std_2: Optional[float] = None, adaptive: Optional[dict] = None) -> torch.Tensor:
-        """CFM sampler (cfm_superresolution.py:162-284 up to `sampled`): prior + fixed-grid ODE (+ mel_pp).
-        std_1 / std_2: the reference falls back to (1.0, sigma) unless BOTH are given (:180-183)."""
+                   std_2: Optional[float] = None, adaptive: Optional[dict] = None, atol: float = 1e-5,
+                   rtol: float = 1e-5, joint: bool = False) -> torch.Tensor:
+        """CFM sampler (cfm_superresolution.py:162-284 up to `sampled`): prior + ODE solve (+ mel_pp).
+        std_1 / std_2: the reference falls back to (1.0, sigma) unless BOTH are given (:180-183).
+        ode_method: torchdiffeq's euler / midpoint / rk4 on the fixed grid linspace(0, 1, steps + 1), or its adaptive
+        dopri5 under atol / rtol, solving the batch as one problem when `joint` (`sample()`) and clip by clip otherwise
+        (`generate*`).  `adaptive` (use_torchode=True) takes priority over ode_method."""
         if std_1 is None or std_2 is None:
             std_1, std_2 = 1.0, float(sigma)
-        if ode_method not in ("euler", "midpoint"):
-            raise ValueError(f"unsupported ODE method {ode_method!r} (euler|midpoint)")
+        rk.check_torchdiffeq_method(ode_method)
         self._chk(cond_mel, eps)
         B, N, Din = cond_mel.shape
         n = cond_mel.numel()
@@ -815,11 +929,17 @@ class Engine:
         if adaptive is not None:  # use_torchode=True (cfm_superresolution.py:259-276): only t_eval[0] / t_eval[-1] matter
             y = self._odeint_adaptive(y, cond_mel, null, cond_scale, float(tgrid[0]), float(tgrid[-1]), **adaptive)
             steps = 0
+        elif ode_method == "dopri5":  # interior grid points are interpolated, never stepped to: only the end points matter
+            y = self._odeint_dopri5(y, cond_mel, null, cond_scale, float(tgrid[0]), float(tgrid[-1]), atol=atol, rtol=rtol,
+                                    joint=joint)
+            steps = 0
         for i in range(steps):
             t0, t1 = tgrid[i], tgrid[i + 1]
             dt = np.float32(t1 - t0)
             if ode_method == "euler":
                 packed = self._field_update(y, cond_mel, null, float(t0), y, float(dt), y, cond_scale, packed)
+            elif ode_method == "rk4":
+                packed = self._rk4_step(y, cond_mel, null, t0, t1, cond_scale, packed)
             else:
                 half = np.float32(0.5) * dt
                 packed = self._field_update(y, cond_mel, null, float(t0), y, float(half), ymid, cond_scale, packed)

@@ -297,6 +297,16 @@ class FlowHighSR(nn.Module):
             return None
         return dict(tableau=self._tableau, atol=float(self.odeint_kwargs["atol"]), rtol=float(self.odeint_kwargs["rtol"]))
 
+    def _host_driven_ode(self) -> bool:
+        """Adaptive solves (torchode, torchdiffeq's dopri5) decide every step on the host: never graph-captured."""
+        return self.use_torchode or self.odeint_kwargs["method"] == "dopri5"
+
+    def _ode(self, joint: bool) -> dict:
+        """ODE arguments of `Engine.sample_mel`.  `joint`: torchdiffeq's adaptive dopri5 solves the batch it is given as
+        one problem (`sample()` with B > 1); the `generate*` paths are per clip like the reference's batch-1 `generate`."""
+        return dict(ode_method=self.odeint_kwargs["method"], atol=float(self.odeint_kwargs["atol"]),
+                    rtol=float(self.odeint_kwargs["rtol"]), adaptive=self._adaptive(), joint=joint)
+
     def _staging(self, numel: int) -> torch.Tensor:
         """Page-locked flat fp32 staging buffer of the batched host path (the clips of a group one after the other), cached
         per size (a few entries, least recently used out).  The previous upload from it must have left the host before it
@@ -347,10 +357,9 @@ class FlowHighSR(nn.Module):
         is_audio = cond.dim() == 2 or (cond.dim() == 3 and cond.shape[1] == 1)
         if is_audio:
             cond = eng.encode(cond.reshape(cond.shape[0], -1))
-        mel = eng.sample_mel(cond, self._noise_like(cond, eps), steps=int(time_steps),
-                             ode_method=self.odeint_kwargs["method"], cfm_method=cfm_method, sigma=float(self.sigma),
-                             cond_scale=float(cond_scale), mel_pp=bool(mel_pp), std_1=float(std_1), std_2=float(std_2),
-                             adaptive=self._adaptive())
+        mel = eng.sample_mel(cond, self._noise_like(cond, eps), steps=int(time_steps), cfm_method=cfm_method,
+                             sigma=float(self.sigma), cond_scale=float(cond_scale), mel_pp=bool(mel_pp), std_1=float(std_1),
+                             std_2=float(std_2), **self._ode(joint=True))
         if not decode_to_audio:
             return mel
         out = eng.vocoder(mel).unsqueeze(1)
@@ -434,7 +443,7 @@ class FlowHighSR(nn.Module):
         for gi, ((T_out, _), idxs) in enumerate(work):
             if check and gi > 0 and out_host is None:
                 flags |= eng.status_read()  # one status word per engine: collect the previous group's before the next resets it
-            graphed = self.cuda_graphs and len(idxs) <= self.cuda_graph_max_batch and not self.use_torchode
+            graphed = self.cuda_graphs and len(idxs) <= self.cuda_graph_max_batch and not self._host_driven_ode()
             # Clips that already sit in page-locked fp32 memory go to the device directly, one asynchronous copy each: no
             # staging copy, and no pass over the samples for the int16 heuristic (flowhighsr.py:62-63) -- dividing by
             # 32768 is an exact power-of-two scaling that the peak normalisation behind the resampler cancels bit for bit
@@ -539,9 +548,8 @@ class FlowHighSR(nn.Module):
             eng.status_begin()
         cond = eng.resample_normalise_parts(parts, target_sr, method=self._resample_method())
         cond_mel = eng.encode(cond)
-        mel = eng.sample_mel(cond_mel, self._noise_like(cond_mel, eps_dev), steps=timestep,
-                             ode_method=self.odeint_kwargs["method"], cfm_method=self.cfm_method, sigma=float(self.sigma),
-                             adaptive=self._adaptive())
+        mel = eng.sample_mel(cond_mel, self._noise_like(cond_mel, eps_dev), steps=timestep, cfm_method=self.cfm_method,
+                             sigma=float(self.sigma), **self._ode(joint=False))
         wave = eng.vocoder(mel)
         if pp_chunk <= 0:
             out = eng.postprocess(wave, cond)
@@ -681,9 +689,8 @@ class FlowHighSR(nn.Module):
             c = chunks[b0: b0 + max_batch]
             mel_c = eng.encode(c)
             e = eps[k0 + b0: k0 + b0 + c.shape[0]]
-            mel = eng.sample_mel(mel_c, self._noise_like(mel_c, e), steps=int(timestep),
-                                 ode_method=self.odeint_kwargs["method"], cfm_method=self.cfm_method,
-                                 sigma=float(self.sigma), adaptive=self._adaptive())
+            mel = eng.sample_mel(mel_c, self._noise_like(mel_c, e), steps=int(timestep), cfm_method=self.cfm_method,
+                                 sigma=float(self.sigma), **self._ode(joint=False))
             waves[b0: b0 + c.shape[0]] = eng.vocoder(mel)
         if world > 1:
             waves = sharding.gather_blocks(waves, per, K, group)  # the only collective of the path
